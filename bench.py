@@ -3,6 +3,7 @@
 QDecoder=16); --config C1..C5 selects the other BASELINE.json configurations (synthetic AWGN frames of each shape).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NS|C1|C2|C3|C4|C5] [--batch F]
+                    [--dump-outputs DIR]
 
 A "step" decodes one batch of F frames per GPU (inputs > L2 so no flush is needed).  Prints ONE JSON line:
   value     decoded frames/s over all GPUs, inputs resident in HBM (pd_decode_device), CUDA-event timed, max over ranks
@@ -14,6 +15,13 @@ A "step" decodes one batch of F frames per GPU (inputs > L2 so no flush is neede
   roofline  algorithmic bytes (N symbols in + K bits out per frame) / kernel time vs measured HBM peak
   cpu_baseline  the compiled reference (oracle/_ref), one process per host core, on a bounded sample (N=1 only)
 `--impl reference` times the reference's own CPU implementation on the same workload instead.
+`--dump-outputs DIR` writes what the last timed step computed, for comparing two builds output for output:
+  decoded_bits.npy  float32 [frames, A], rank 0's frames only: a fixed seeded sample of the batch that rank 0 decoded in
+                    the step (all of it when it fits in 56 MB)
+  frame_index.npy   float64 [frames], the rows of rank 0's batch that decoded_bits holds
+  error_counts.npy  float64 [2], bit errors and block errors of the step summed over ALL GPUs (with --gpus 1: over the
+                    whole batch, not just the sampled rows)
+The inputs depend only on the arguments (seeded per rank), so two runs with the same arguments decode the same frames.
 Multi-GPU: one process per GPU (torchrun); frames are sharded, no data-path collective; the only exchange is the
 NCCL all-reduce of the two error counters (bit / block errors), inside the timed region.
 """
@@ -31,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 PKG = os.path.join(ROOT, "quantized_decoder_polar_codes_b200")
 
 
@@ -377,11 +386,12 @@ def run_ours(args, rank, local_rank, world):
     cnt = counters.cpu().tolist()
     total_frames = world * F * args.steps
     ref_out = d_out.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ref_out, step_cnt.cpu().numpy())
     note(f"device-resident: {value:.4g} frames/s")
 
     # --- end to end (1), `e2e`: the reference-facing call -- decode((B,N) array) of the pybind class -- on input in pinned host
     #     memory in the compact dtype (uint8 symbols / float64 LLRs), result a fresh numpy array; H2D and D2H copies inside ---
-    e2e_steps = max(2, min(args.steps, 10))
     h_in_p = lib.pd_host_alloc(F * N * esz)
     h_out_p = lib.pd_host_alloc(F * Kout)
     h_in = np.ctypeslib.as_array(ctypes.cast(h_in_p, ctypes.POINTER(ctypes.c_uint8 if lut else ctypes.c_double)), (F, N))
@@ -391,10 +401,10 @@ def run_ours(args, rank, local_rank, world):
         got = dec.decode(h_in)
     barrier()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         got = dec.decode(h_in)
     e2e_s = time.perf_counter() - t0
-    e2e_value = world * F * e2e_steps / D.max_over_ranks(e2e_s, dev)
+    e2e_value = world * F * args.steps / D.max_over_ranks(e2e_s, dev)
     same = bool((got == ref_out).all())
     note(f"e2e through decode() on pinned input: {e2e_value:.4g} frames/s")
 
@@ -405,10 +415,10 @@ def run_ours(args, rank, local_rank, world):
         got = dec.decode(x_api)
     barrier()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         got = dec.decode(x_api)
     e2e_api_s = time.perf_counter() - t0
-    e2e_api = world * F * e2e_steps / D.max_over_ranks(e2e_api_s, dev)
+    e2e_api = world * F * args.steps / D.max_over_ranks(e2e_api_s, dev)
     same_api = bool((got == ref_out).all())
     del x_api
     note(f"e2e through decode() as the drivers call it: {e2e_api:.4g} frames/s")
@@ -418,11 +428,11 @@ def run_ours(args, rank, local_rank, world):
         capi.decode_host(dec, h_in_p, pd_dtype, F, h_out_p)
     barrier()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         capi.decode_host(dec, h_in_p, pd_dtype, F, h_out_p)
     torch.cuda.synchronize()
     e2e_c_s = time.perf_counter() - t0
-    e2e_cabi = world * F * e2e_steps / D.max_over_ranks(e2e_c_s, dev)
+    e2e_cabi = world * F * args.steps / D.max_over_ranks(e2e_c_s, dev)
     same = same and bool((h_out == ref_out).all())
     del h_in, h_out
     lib.pd_host_free(h_in_p)
@@ -479,6 +489,21 @@ def run_ours(args, rank, local_rank, world):
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 56 << 20     # decoded_bits.npy stays below this; the two small arrays fit in the rest of 64 MB
+
+
+def dump_outputs(path, bits, step_counts):
+    """decoded bits of the last timed step (a seeded sample of its frames when the batch is larger than DUMP_BYTES allows)
+    and that step's error counters, as float .npy files under `path`"""
+    F, A = bits.shape
+    n = min(F, DUMP_BYTES // (4 * A))
+    rows = np.arange(F) if n == F else np.sort(np.random.default_rng(0).choice(F, n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "decoded_bits.npy"), bits[rows].astype(np.float32))
+    np.save(os.path.join(path, "frame_index.npy"), rows.astype(np.float64))
+    np.save(os.path.join(path, "error_counts.npy"), np.asarray(step_counts, np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -509,7 +534,13 @@ def main():
     ap.add_argument("--ref-frames", type=int, default=0, help="CPU reference: frames per core per step (default: a few seconds of work)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--verbose", action="store_true", help="progress notes on stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm keeps no outputs)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

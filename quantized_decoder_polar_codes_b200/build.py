@@ -77,12 +77,25 @@ def build_cuda(force=False, verbose=False):
     return LIB
 
 
+def pybind11_include():
+    """pybind11's header directory: the pybind11 package's, else the copy torch ships (torch is a dependency anyway, so a
+    Python environment without the pybind11 package still builds)"""
+    try:
+        import pybind11
+        return pybind11.get_include()
+    except ImportError:
+        import torch
+        inc = os.path.join(os.path.dirname(torch.__file__), "include")
+        if not os.path.isfile(os.path.join(inc, "pybind11", "pybind11.h")):
+            raise RuntimeError("pybind11 headers not found: neither the pybind11 package nor torch's copy is installed")
+        return inc
+
+
 def build_pybind(force=False):
     src = os.path.join(CSRC, "pb_pybind.cpp")
     if force or _newer(EXT, [src, os.path.join(ROOT, "include", "polar_b200.h"), LIB]):
-        import pybind11
         cmd = ["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-fvisibility=hidden",
-               "-I" + sysconfig.get_paths()["include"], "-I" + pybind11.get_include(), src,
+               "-I" + sysconfig.get_paths()["include"], "-I" + pybind11_include(), src,
                "-L" + HERE, "-lpolar_b200", "-Wl,-rpath,$ORIGIN", "-o", EXT]
         subprocess.check_call(cmd)
     return EXT

@@ -6,8 +6,8 @@ quantized_decoder_polar_codes_b200.run_driver (compat shims: numpy, torchtracer,
 generator's layout, with the compiled reference's decoders behind the PolarDecoder import path -- and the restated loop of
 tests/driver_loop.py, same seed, ends with the same error counters.  That pins the restated loop to the script.
 GPU: the restated loop from the same pickles with THIS package behind every import the script makes (PolarDecoder.Decoder.*,
-PolarBDEnc.Encoder.*, quantizers.quantizer.LLROptLSQuantizer) against the compiled reference's decoders: every decoded word
-and therefore BER/BLER identical."""
+PolarBDEnc.Encoder.*, quantizers.quantizer.LLROptLSQuantizer) against the compiled reference's decoders (the oracle's where
+the reference is not built): every decoded word and therefore BER/BLER identical."""
 import os
 import sys
 import types
@@ -133,9 +133,16 @@ def test_compat_numpy_shims():
 # ---------------------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
 @pytest.mark.parametrize("decoder_type,is_crc", [("SC-LUT", False), ("SCL-LUT", False), ("FastSC-LUT", False), ("FastSCL-LUT", False), ("CASCL-LUT", True)])
-def test_driver_loop_on_this_package_equals_the_reference(workdir, refmod, decoder_type, is_crc):
-    """what the script would do with this package installed: same pickles, same seed, every import served by the package"""
+def test_driver_loop_on_this_package_equals_the_reference(workdir, decoder_type, is_crc):
+    """what the script would do with this package installed: same pickles, same seed, every import served by the package.
+    The other side is the compiled reference's decoders where it has been built.  Without it they are oracle decoders whose
+    positional arguments are named by test_abi.REF_SIGNATURES, the reference's constructor signatures as transcribed from its
+    sources; only test_reference_signatures_agree_with_compiled_reference, which needs the reference, checks that
+    transcription.  On the LLR-domain tables used here the oracle's decoded words are pinned to the reference's by
+    tests/golden/real_lut_n128.npz."""
+    from oracle import polar_oracle as po
     from quantized_decoder_polar_codes_b200 import lutgen
+    from test_abi import REF_SIGNATURES
     compat.install()
     import importlib
     ours = {k: getattr(importlib.import_module("PolarDecoder.Decoder." + k), k)
@@ -143,7 +150,11 @@ def test_driver_loop_on_this_package_equals_the_reference(workdir, refmod, decod
     PolarEnc = importlib.import_module("PolarBDEnc.Encoder.PolarEnc").PolarEnc
     CRCEnc = importlib.import_module("PolarBDEnc.Encoder.CRCEnc").CRCEnc
     LLRQuantizer = importlib.import_module("quantizers.quantizer.LLROptLSQuantizer").LLRQuantizer
-    ref = {k: getattr(refmod, k) for k in ours}
+    refmod = po.load_reference()
+    if refmod is not None:
+        ref = {k: getattr(refmod, k) for k in ours}
+    else:
+        ref = {k: (lambda *a, k=k: po.OracleDecoder(k, **dict(zip(REF_SIGNATURES[k], a)))) for k in ours}
     frames, seed, A = 60, 11, 32
     args = (workdir, N, A, 8, decoder_type, is_crc, QCU, QD, QC, DESIGN, frames, seed, [0, 2, 4])
     s1, w1 = driver_loop.run(*args, ours, PolarEnc, CRCEnc, LLRQuantizer, pw_sets, node_types, lutgen.channel_llr_density_table)
