@@ -39,7 +39,7 @@ def _sources(exts):
 # translation units of libpolar_b200.so: (object name, source, extra flags, headers it depends on besides its source)
 _COMMON = ["pb_internal.h", "pb_generic.cuh"]
 _UNITS = [("capi", "pb_capi.cu", [], None)]          # None = every header
-_UNITS += [("k%d" % t, "pb_kernels.cu", ["-DPB_TU=%d" % t], _COMMON + ["pb_scl_lut.cuh"]) for t in (1, 2, 3, 4, 11, 12, 13, 14)]
+_UNITS += [("k%d" % t, "pb_kernels.cu", ["-DPB_TU=%d" % t], _COMMON + ["pb_scl_lut.cuh"]) for t in (1, 2, 3, 4)]
 _UNITS += [("k%d" % t, "pb_kernels.cu", ["-DPB_TU=%d" % t], _COMMON + ["pb_path_warp.cuh"]) for t in (5, 6, 7, 8)]
 _UNITS += [("k9", "pb_kernels.cu", ["-DPB_TU=9"], _COMMON)]
 _UNITS += [("lutgen", "pb_lutgen.cu", [], ["pb_lutgen.cuh"])]

@@ -41,10 +41,6 @@ const void *scl_fn_l3_plain(bool ca);
 const void *scl_fn_l3_fast(bool ca);
 const void *scl_fn_l01(int logL, bool ca, bool fast);
 const void *scl_fn_l2(bool ca, bool fast);
-const void *scl_fn_l3_plain_priv(bool ca);
-const void *scl_fn_l3_fast_priv(bool ca);
-const void *scl_fn_l01_priv(int logL, bool ca, bool fast);
-const void *scl_fn_l2_priv(bool ca, bool fast);
 const void *path_fn_lut(int logL);
 const void *path_fn_float(int logL);
 const void *path_fn_uniform(int logL);
@@ -56,12 +52,7 @@ cudaError_t launch_optls(int n_problems, size_t smem, const double *density, con
 cudaError_t launch_mmi_table(int P, int M, int W, int mode, const double *p1, const double *p2, const double *l1, const double *l2,
                              double c1, double c2, double *out1, double *out2);
 cudaError_t launch_mmi_dp(int P, int M, int K, int W, const double *T, int32_t *lm, int32_t *Az);
-const void *fast_kernel_fn(int logL, bool ca, bool fast, bool priv) {
-    if (priv) {
-        if (logL >= 3) return fast ? scl_fn_l3_fast_priv(ca) : scl_fn_l3_plain_priv(ca);
-        if (logL == 2) return scl_fn_l2_priv(ca, fast);
-        return scl_fn_l01_priv(logL, ca, fast);
-    }
+const void *fast_kernel_fn(int logL, bool ca, bool fast) {
     if (logL >= 3) return fast ? scl_fn_l3_fast(ca) : scl_fn_l3_plain(ca);
     if (logL == 2) return scl_fn_l2(ca, fast);
     return scl_fn_l01(logL, ca, fast);
@@ -318,7 +309,6 @@ struct pd_decoder {
     size_t ws_user_cap = 0;
     StreamSlot slot[2];
     int64_t chunk_frames = 0;
-    int grid_div = 1;         // pd_decode_device, split batches: 2 = each concurrent launch takes half of the CTA slots (experiment knob)
     // pd_decode, tiny calls (the reference drivers decode one frame per call): a mapped pinned staging area the kernel
     // reads and writes directly -- no copy engine round trips
     char *h_small = nullptr, *d_small = nullptr;
@@ -534,7 +524,7 @@ bool want_path(const pd_decoder *D, int dtype, const void *d_in) {
 int launch(pd_decoder *D, const void *d_in, int dtype, int64_t B, uint8_t *d_out, cudaStream_t s, char *ws) {
     if (B <= 0) return PD_OK;
     if (want_fast(D, dtype, d_in)) {
-        int rc = launch_fast_lut(D->dev, D->fast, d_in, dtype, B, d_out, s, reinterpret_cast<uint32_t *>(ws), D->d_err, D->dbg_pm, D->dbg_win, std::max(1, D->sm_count / D->grid_div));
+        int rc = launch_fast_lut(D->dev, D->fast, d_in, dtype, B, d_out, s, reinterpret_cast<uint32_t *>(ws), D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
         g_launches++;
         if (rc != 0) return fail(PD_ECUDA, "fast kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc));
         return PD_OK;
@@ -826,10 +816,10 @@ int pd_decode_device(pd_decoder *D, const void *dev_in, int in_dtype, int64_t B,
     if (B <= 0) return PD_OK;
     CUDA_TRY(cudaSetDevice(D->device));
     cudaStream_t s = (cudaStream_t)cuda_stream;
-    // One launch per call for the plain scl_lut_warp kernels with the private ring: their warps take frame groups from a
-    // counter, so the launch has no tail, and one value workspace (72 MB at N=1024, L=8) stays L2-resident.
-    // Every other persistent kernel (static schedule: path_warp, the shared-ring variants; and the Fast-SSC variants, which
-    // are instruction-fetch bound and run 30 % faster when the warps of an SM start their walks together) gets its batch in
+    // One launch per call for the plain scl_lut_warp kernels: their warps take frame groups from a counter, so the launch
+    // has no tail, and one value workspace (72 MB at N=1024, L=8) stays L2-resident.
+    // The other persistent kernels (path_warp, with its static schedule, and the Fast-SSC variants of scl_lut_warp, which
+    // are instruction-fetch bound and run 30 % faster when the warps of an SM start their walks together) get their batch in
     // pieces of ONE wave, issued alternately on two internal streams forked from / joined to the caller's stream with
     // events: the CTAs of piece k+1 move into the slots that the CTAs of piece k vacate, so nothing idles between pieces.
     // POLAR_B200_FORCE_SPLIT=0/1 overrides, POLAR_B200_PIECE_WAVES sets the piece size.
@@ -837,7 +827,7 @@ int pd_decode_device(pd_decoder *D, const void *dev_in, int in_dtype, int64_t B,
     const int64_t wave = wave_frames(D, in_dtype, dev_in);
     static const int force_split = getenv("POLAR_B200_FORCE_SPLIT") ? atoi(getenv("POLAR_B200_FORCE_SPLIT")) : -1;
     static const int piece_waves = getenv("POLAR_B200_PIECE_WAVES") ? std::max(1, atoi(getenv("POLAR_B200_PIECE_WAVES"))) : 1;
-    const bool dynamic_kernel = want_fast(D, in_dtype, dev_in) && D->fast.p.priv && !D->fast.fastk;
+    const bool dynamic_kernel = want_fast(D, in_dtype, dev_in) && !D->fast.fastk;
     const bool split = force_split == 0 ? false
                                         : ((force_split == 1 || !dynamic_kernel) && wave > 0 && B >= 2 * wave * piece_waves && ((N * esz) % 16 == 0));
     const int64_t per = split ? wave * piece_waves : B;
@@ -865,20 +855,14 @@ int pd_decode_device(pd_decoder *D, const void *dev_in, int in_dtype, int64_t B,
     // Both pieces in flight use a full grid and their own value workspace (2 x 52 MB at N=1024, L=8): together with the
     // streaming input / output that exceeds the 126 MB L2, so part of the workspace is written back and re-read (ncu,
     // --cache-control none: 5.2 KB of DRAM traffic per frame vs 1.5 KB algorithmic = 65 GB/s, 1 % of the HBM peak).
-    // POLAR_B200_HALF_GRID_PIECES=1 gives each piece half of the CTA slots instead: traffic 2.2 KB/frame, but 10 % fewer
-    // frames/s (the pieces no longer back-fill each other's tails) -- measured, not the default.
-    D->grid_div = getenv("POLAR_B200_HALF_GRID_PIECES") ? 2 : 1;
     for (int pc = 0; pc < pieces; ++pc) {
         const int64_t f0 = (int64_t)pc * per, nb = std::min<int64_t>(per, B - f0);
         if (nb <= 0) break;
         const int w = pc & 1;
         if ((rc = launch(D, (const char *)dev_in + (size_t)f0 * N * esz, in_dtype, nb, dev_out + (size_t)f0 * Ko, D->side[w],
-                         D->ws_user ? D->ws_user + (size_t)w * need1 : nullptr))) {
-            D->grid_div = 1;
+                         D->ws_user ? D->ws_user + (size_t)w * need1 : nullptr)))
             return rc;
-        }
     }
-    D->grid_div = 1;
     for (int i = 0; i < 2; ++i) {
         CUDA_TRY(cudaEventRecord(D->join_ev[i], D->side[i]));
         CUDA_TRY(cudaStreamWaitEvent(s, D->join_ev[i], 0));
@@ -890,12 +874,6 @@ int pd_check(pd_decoder *D, void *cuda_stream) {
     if (!D) return fail(PD_EINVAL, "null decoder");
     CUDA_TRY(cudaSetDevice(D->device));
     CUDA_TRY(cudaStreamSynchronize((cudaStream_t)cuda_stream));
-    if (*D->h_err & 0x40000000) {      // POLAR_B200_NO_TMA=2 (debug): a ring chunk differed from the stream
-        const int v = *D->h_err;
-        *D->h_err = 0;
-        return fail(PD_ECUDA, "ring check: chunk %d warp %d lane %d differs from the stream%s%s", v & 0xffff, (v >> 16) & 7, (v >> 19) & 31,
-                    (v & 0x20000000) ? " [holds the previous round's chunk: read too early]" : "", (v & 0x10000000) ? " [holds the next round's chunk: overwritten too early]" : "");
-    }
     if (*D->h_err) {
         *D->h_err = 0;
         return fail(PD_ERANGE, "an input symbol is outside the root lookup table (valid: [0,%d) for the first half, [0,%d) for the second)", D->dev.root_qa, D->dev.root_qb);

@@ -4,28 +4,19 @@
 //         2  scl_lut_warp L=8 Fast-SSC variants      6  path_warp float
 //         3  scl_lut_warp L=1,2                      7  path_warp uniform
 //         4  scl_lut_warp L=4                        8  path_warp Lloyd
-//     11-14  = 1-4 with the private per-warp table ring (POLAR_B200_RING=private)
-#if (PB_TU >= 1 && PB_TU <= 4) || (PB_TU >= 11 && PB_TU <= 14)
+#if PB_TU >= 1 && PB_TU <= 4
 #define PB_TU_SCL
 #include "pb_scl_lut.cuh"
 namespace pb {
-// PB_TU 11..14 = the same families with the private per-warp cp.async ring (PRIV) instead of the CTA-shared TMA ring
-#if PB_TU > 10
-#define PB_SCL_FN(name) name##_priv
-constexpr bool kPriv = true;
+#if PB_TU == 1
+const void *scl_fn_l3_plain(bool ca) { return fast_kernel_fn_l<3, false>(ca); }
+#elif PB_TU == 2
+const void *scl_fn_l3_fast(bool ca) { return fast_kernel_fn_l<3, true>(ca); }
+#elif PB_TU == 3
+const void *scl_fn_l01(int logL, bool ca, bool fast) { if (logL == 0) return fast ? fast_kernel_fn_l<0, true>(false) : fast_kernel_fn_l<0, false>(false);
+    return fast ? fast_kernel_fn_l<1, true>(ca) : fast_kernel_fn_l<1, false>(ca); }
 #else
-#define PB_SCL_FN(name) name
-constexpr bool kPriv = false;
-#endif
-#if PB_TU % 10 == 1
-const void *PB_SCL_FN(scl_fn_l3_plain)(bool ca) { return fast_kernel_fn_l<3, false, kPriv>(ca); }
-#elif PB_TU % 10 == 2
-const void *PB_SCL_FN(scl_fn_l3_fast)(bool ca) { return fast_kernel_fn_l<3, true, kPriv>(ca); }
-#elif PB_TU % 10 == 3
-const void *PB_SCL_FN(scl_fn_l01)(int logL, bool ca, bool fast) { if (logL == 0) return fast ? fast_kernel_fn_l<0, true, kPriv>(false) : fast_kernel_fn_l<0, false, kPriv>(false);
-    return fast ? fast_kernel_fn_l<1, true, kPriv>(ca) : fast_kernel_fn_l<1, false, kPriv>(ca); }
-#else
-const void *PB_SCL_FN(scl_fn_l2)(bool ca, bool fast) { return fast ? fast_kernel_fn_l<2, true, kPriv>(ca) : fast_kernel_fn_l<2, false, kPriv>(ca); }
+const void *scl_fn_l2(bool ca, bool fast) { return fast ? fast_kernel_fn_l<2, true>(ca) : fast_kernel_fn_l<2, false>(ca); }
 #endif
 }  // namespace pb
 #elif PB_TU >= 5 && PB_TU <= 8
@@ -60,5 +51,5 @@ const void *generic_kernel_fn(int dom, bool l, bool w) {
 }
 }  // namespace pb
 #else
-#error "PB_TU must be 1..9 or 11..14"
+#error "PB_TU must be 1..9"
 #endif

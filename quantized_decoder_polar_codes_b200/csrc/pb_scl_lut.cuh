@@ -13,14 +13,11 @@
 //   * f / g lookups: the 16x16 nibble table of the node is ONE 32-bit register per lane (128 B per warp) and a
 //     lookup is a warp shuffle + shift (no bank conflicts, no shared memory);
 //   * every table / LLR row is consumed exactly once per pass and in a fixed order, so the host lays them out
-//     as one linear stream of 128-byte lines.  Two ways to bring it on chip (template parameter PRIV):
-//     a private 4-chunk ring per warp that every lane fills with cp.async (default), or one ring per CTA that a
-//     producer warp fills with TMA bulk copies + mbarriers (POLAR_B200_RING=shared; see DESIGN.md 4.1 for why it
-//     is not the default);
+//     as one linear stream of 128-byte lines, which every warp brings on chip through a private 4-chunk ring that
+//     its lanes fill with cp.async;
 //   * fork: 2L path metrics ranked with a stable (key,index) count -- identical to libstdc++'s insertion sort
 //     for 2L <= 16 (PD/src/SCLLUTDecoder.cpp:8-22, SURVEY App. B1);
-//   * schedule: persistent CTAs of 4 warps; the PRIV kernels take frame groups from a counter in the workspace
-//     (dynamic), the shared-ring kernels walk a static schedule;
+//   * schedule: persistent CTAs of 4 warps that take frame groups from a counter in the workspace (dynamic);
 //   * code size matters as much as instruction count: an SM's warps sit all over the walk, the instruction cache
 //     sees the whole kernel (DESIGN.md 4.1).
 // Output: the root partial sums x of the selected path are turned back into u = x F^{(x)n} and gathered.
@@ -39,22 +36,9 @@
 #include "pb_generic.cuh"
 #include "pb_internal.h"
 
-#ifndef PB_DEFAULT_RING_PRIVATE
-#define PB_DEFAULT_RING_PRIVATE true      // which table ring plan_fast_lut picks when POLAR_B200_RING is not set
-#endif
-#ifndef PB_EXP_LINE
-#define PB_EXP_LINE 0
-#endif
-
 namespace pb {
 
-// Table stream ring, one per CTA, filled by the producer warp with TMA bulk copies (cp.async.bulk + mbarrier):
-// kStages stages of kCPS chunks (512 bytes = 4 table lines, lane-transposed) each.
-constexpr int kStages = 4;
-constexpr int kCPS = 4;
-constexpr int kRingSlots = kStages * kCPS;          // chunks in the ring
-constexpr unsigned kStageBytes = kCPS * 512u;
-constexpr int kMaxWarps = 4;                         // decoding warps per CTA (+ 1 producer warp in the shared-ring kernels)
+constexpr int kMaxWarps = 4;                         // decoding warps per CTA
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kWsHeadWords = 64;                     // launch state at the head of the workspace (256 bytes)
 
@@ -74,11 +58,12 @@ struct FastParams {
     int r1_words;                  // shared-memory words for the R1 scratch (0 when the code has no R1 node)
     const uint32_t *crc_rem;       // [A] CRC remainder of each unit message bit (CA kinds)
     uint32_t crc_checkmask;
-    int warps;                     // consumer warps per CTA; one more warp streams the tables
+    int warps;                     // decoding warps per CTA
     int dbg;                       // POLAR_B200_KDEBUG: 1 = never take the sorted-keeps shortcut in fork (A/B measurements)
-    int priv;                      // the kernel is a PRIV instantiation (private per-warp rings, no producer warp)
-    int no_tma;                    // debug knob (POLAR_B200_NO_TMA): the producer warp copies the stages with plain loads / stores
-    int warp_words;                // shared-memory words of one consumer warp (its V, X, scratch, fork cells)
+    int reserved[2];               // unused: keeps the offsets of the fields below, which the kernels' register allocation
+                                   // (and so the occupancy and pd_wave_frames) follows -- without it the L=1 kernel of
+                                   // SCLUTDecoder drops from 61 to 56 registers and gets a different wave size
+    int warp_words;                // shared-memory words of one decoding warp (its V, X, scratch, fork cells)
     int vwords, xwords, scrwords;  // shared-memory words per lane: value levels gl+1..top, X; scratch words per warp
     int scr_off;                   // word offset of the epilogue scratch: its own region, or 0 = on top of the (then dead) value levels
     int gl;                        // value levels 1..gl live in the global (L2-resident) workspace, the rest in shared memory
@@ -105,21 +90,6 @@ struct FastPlan {
 #ifdef PB_HOST_EMU
 using smaddr_t = size_t;
 __device__ __forceinline__ uint4 lds128(smaddr_t a) { uint4 v; memcpy(&v, reinterpret_cast<const void *>(a), 16); return v; }
-// mbarrier: {arrivals still pending, arrivals per phase, completed phases}
-struct EmuBar { uint16_t pending, count; uint32_t phases; };
-__device__ __forceinline__ void mbar_init(smaddr_t b, unsigned count) { *reinterpret_cast<EmuBar *>(b) = EmuBar{(uint16_t)count, (uint16_t)count, 0u}; }
-__device__ __forceinline__ void mbar_fence_init() {}
-__device__ __forceinline__ void mbar_arrive(smaddr_t b) {
-    EmuBar *m = reinterpret_cast<EmuBar *>(b);
-    if (--m->pending == 0) { m->pending = m->count; m->phases++; }
-}
-__device__ __forceinline__ void mbar_wait(smaddr_t b, unsigned parity) {   // returns once the phase of that parity is complete
-    while ((reinterpret_cast<EmuBar *>(b)->phases & 1u) == parity) pb_emu::yield();
-}
-__device__ __forceinline__ void bulk_load(smaddr_t dst, const void *gsrc, unsigned bytes, smaddr_t bar) {
-    memcpy(reinterpret_cast<void *>(dst), gsrc, bytes);
-    mbar_arrive(bar);
-}
 #else
 using smaddr_t = unsigned;
 __device__ __forceinline__ uint4 lds128(smaddr_t a) {
@@ -127,34 +97,11 @@ __device__ __forceinline__ uint4 lds128(smaddr_t a) {
     asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];\n" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
     return v;
 }
-__device__ __forceinline__ void mbar_init(smaddr_t b, unsigned count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(b), "r"(count)); }
-__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive(smaddr_t b) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(b) : "memory"); }
-__device__ __forceinline__ void mbar_wait(smaddr_t b, unsigned parity) {   // returns once the phase of that parity is complete
-    // (the third operand is a suspend-time hint: the waiting warp sleeps in hardware instead of spinning on issue slots)
-    asm volatile("{\n .reg .pred p;\n WAIT_%=:\n mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n @p bra DONE_%=;\n bra WAIT_%=;\n DONE_%=:\n}\n"
-                 ::"r"(b), "r"(parity), "r"(0x989680u) : "memory");
-}
-// one TMA bulk copy global -> shared; `bar` receives the single arrival and the byte count
-__device__ __forceinline__ void bulk_load(smaddr_t dst, const void *gsrc, unsigned bytes, smaddr_t bar) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(bar), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(dst), "l"(gsrc), "r"(bytes), "r"(bar) : "memory");
-}
-// experiment (POLAR_B200_NO_TMA=3): the .shared::cta destination form, issued by the lane elect.sync picks
-__device__ __forceinline__ void bulk_load_cta(smaddr_t dst, const void *gsrc, unsigned bytes, smaddr_t bar) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(bar), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cta.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(dst), "l"(gsrc), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {
-    unsigned p;
-    asm volatile("{\n .reg .pred q;\n elect.sync _|q, 0xffffffff;\n selp.u32 %0, 1, 0, q;\n}\n" : "=r"(p));
-    return p != 0;
-}
 #endif
 
-// Private ring (PRIV kernels): every lane copies ITS 16 bytes of a chunk with cp.async into a ring owned by its warp -- no
-// barrier, no producer warp; kPrivChunks - 1 chunks in flight per lane.
-constexpr int kPrivChunks = 4;
+// Table ring: every lane copies ITS 16 bytes of a chunk (512 bytes = 4 table lines, lane-transposed) with cp.async into a
+// ring owned by its warp -- no barrier, nothing shared between warps; kRingChunks - 1 chunks in flight per lane.
+constexpr int kRingChunks = 4;
 #ifdef PB_HOST_EMU
 __device__ __forceinline__ void cp_async16(smaddr_t dst, const void *gsrc) { memcpy(reinterpret_cast<void *>(dst), gsrc, 16); }
 template <int NPEND> __device__ __forceinline__ void cp_async_wait() {}
@@ -165,19 +112,20 @@ __device__ __forceinline__ void cp_async16(smaddr_t dst, const void *gsrc) {
 template <int NPEND> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(NPEND) : "memory"); }
 #endif
 // `fetch` = byte offset (inside the lane's column of the stream) of the next chunk to request; wraps at the end of the stream
-__device__ __forceinline__ uint4 priv_next_chunk(uint32_t &cc, uint32_t &fetch, smaddr_t ring_lane, const char *stream_lane, uint32_t stream_bytes) {
-    const uint32_t slot = cc & (kPrivChunks - 1);
-    cp_async16(ring_lane + ((slot + kPrivChunks - 1) & (kPrivChunks - 1)) * 512u, stream_lane + fetch);   // refill the slot consumed before
+__device__ __forceinline__ uint4 ring_next_chunk(uint32_t &cc, uint32_t &fetch, smaddr_t ring_lane, const char *stream_lane, uint32_t stream_bytes) {
+    const uint32_t slot = cc & (kRingChunks - 1);
+    cp_async16(ring_lane + ((slot + kRingChunks - 1) & (kRingChunks - 1)) * 512u, stream_lane + fetch);   // refill the slot consumed before
     fetch += 512u;
     if (fetch == stream_bytes) fetch = 0u;
-    cp_async_wait<kPrivChunks - 1>();                                                                     // ... and make sure this chunk has landed
+    cp_async_wait<kRingChunks - 1>();                                                                     // ... and make sure this chunk has landed
     ++cc;
     return lds128(ring_lane + slot * 512u);
 }
-static __device__ __noinline__ uint4 priv_fetch_outlined(uint32_t cc, uint32_t fetch, smaddr_t ring_lane, const char *stream_lane) {
-    const uint32_t slot = cc & (kPrivChunks - 1);
-    cp_async16(ring_lane + ((slot + kPrivChunks - 1) & (kPrivChunks - 1)) * 512u, stream_lane + fetch);
-    cp_async_wait<kPrivChunks - 1>();
+// out-of-line form for the Fast-SSC kernels (~40 consumption sites); the caller advances cc and fetch
+static __device__ __noinline__ uint4 ring_fetch_outlined(uint32_t cc, uint32_t fetch, smaddr_t ring_lane, const char *stream_lane) {
+    const uint32_t slot = cc & (kRingChunks - 1);
+    cp_async16(ring_lane + ((slot + kRingChunks - 1) & (kRingChunks - 1)) * 512u, stream_lane + fetch);
+    cp_async_wait<kRingChunks - 1>();
     return lds128(ring_lane + slot * 512u);
 }
 
@@ -194,27 +142,9 @@ struct R1Less {
 };
 static __device__ __noinline__ void sort_r1_packed(unsigned short *col, int n) { std_sort_acc<16>(R1Acc{col}, n, R1Less{}); }
 
-// Consumer side of the stream ring.  `cc` counts the chunks this warp has consumed since the kernel started; the ring slot,
-// the stage and the barrier phase follow from it.  The first chunk of a stage waits for the stage's "full" barrier, the last
-// one hands the stage back ("empty", one arrival per consumer warp).
-__device__ __forceinline__ uint4 ring_next_chunk(uint32_t &cc, smaddr_t ring_lane, smaddr_t bars, int lane) {
-    const uint32_t slot = cc & (kRingSlots - 1), st = slot / kCPS;
-    if ((cc & (kCPS - 1)) == 0) mbar_wait(bars + st * 8u, (cc / kRingSlots) & 1u);
-    const uint4 v = lds128(ring_lane + slot * 512u);
-    if ((cc & (kCPS - 1)) == kCPS - 1) {
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bars + (kStages + st) * 8u);
-    }
-    ++cc;
-    return v;
-}
-// out-of-line variant for the Fast-SSC kernels (~40 consumption sites)
-static __device__ __noinline__ uint4 ring_fetch_outlined(uint32_t cc, smaddr_t ring_lane, smaddr_t bars, int lane) {
-    return ring_next_chunk(cc, ring_lane, bars, lane);
-}
 struct LineState {
     uint32_t cc;   // chunks consumed so far
-    uint32_t fetch;   // PRIV: stream offset of the next chunk to request
+    uint32_t fetch;   // stream offset of the next chunk to request
     uint4 cur;     // the chunk lines are currently taken from
     int q;         // next line inside `cur` (4 = exhausted)
 };
@@ -224,11 +154,11 @@ __device__ __forceinline__ uint32_t pack4(uint32_t x) {
     return (x & 0xfu) | ((x >> 4) & 0xf0u) | ((x >> 8) & 0xf00u) | ((x >> 12) & 0xf000u);
 }
 
-// One CTA = fp.warps decoding warps, each working on its own frame groups (PRIV: 7 CTAs of 4 warps per SM at N=1024, L=8 =
+// One CTA = fp.warps decoding warps, each working on its own frame groups (7 CTAs of 4 warps per SM at N=1024, L=8 =
 // 28 decoding warps, 72 registers per thread at most; the Fast variants, which run best with 12 resident warps, may take
-// 100), plus -- shared-ring kernels only -- one producer warp that streams the tables (6 CTAs of 4+1 warps, 64 registers).
-template <int LOGL, bool CA, bool FAST, bool PRIV>
-__global__ void __launch_bounds__((kMaxWarps + (PRIV ? 0 : 1)) * 32, PRIV ? (FAST ? 5 : 7) : (FAST ? 4 : 6))
+// 100).
+template <int LOGL, bool CA, bool FAST>
+__global__ void __launch_bounds__(kMaxWarps * 32, FAST ? 5 : 7)
 scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastParams fp, const void *__restrict__ in, int in_dtype,
                     uint8_t *__restrict__ out, long long B, uint32_t *__restrict__ ws, int *err_flag, double *dbg_pm, int *dbg_win) {
     constexpr int L = 1 << LOGL;
@@ -242,80 +172,12 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
 
     // ---- table stream.  Every f/g table (one 128-byte line = 16x16 nibbles) and every leaf LLR row (16 doubles) is
     //      consumed exactly once per pass, in a fixed order, the same for every warp, and lane l only ever needs word l of
-    //      a line.  The host lays the lines out in consumption order, 4 lines per lane-transposed 512-byte chunk; the
-    //      producer warp moves them stage by stage into the CTA's ring with TMA bulk copies, the consumer warps read their
-    //      16 bytes per chunk with one LDS.128.  full[s] / empty[s] mbarriers carry the hand-over. ----
-    //      PRIV kernels: no producer warp and no barriers; each warp keeps a private ring that its lanes fill with
-    //      cp.async (priv_next_chunk).
-    uint32_t *RINGB = sm + (size_t)W * fp.warp_words + (PRIV ? (size_t)wid * (kPrivChunks * 128) : (size_t)0);
+    //      a line.  The host lays the lines out in consumption order, 4 lines per lane-transposed 512-byte chunk; each
+    //      warp keeps a private ring of kRingChunks chunks that its lanes fill with cp.async and read with one LDS.128
+    //      per chunk (ring_next_chunk). ----
+    uint32_t *RINGB = sm + (size_t)W * fp.warp_words + (size_t)wid * (kRingChunks * 128);
     const smaddr_t ring0 = (smaddr_t)__cvta_generic_to_shared(RINGB);
-    const smaddr_t bars = ring0 + kRingSlots * 512u;          // full[kStages], empty[kStages]
-    if (!PRIV) {
-        if (threadIdx.x == 0) {
-            for (int i = 0; i < kStages; ++i) { mbar_init(bars + i * 8u, 1u); mbar_init(bars + (kStages + i) * 8u, (unsigned)W); }
-            mbar_fence_init();
-        }
-        __syncthreads();
-    }
-    // static schedule: in pass p, warp w of CTA b decodes frame group (p * gridDim.x + b) * W + w; a CTA runs as many
-    // passes as its warp 0 has groups (warps without a group still drain the stream)
     const long long n_groups = (B + FPW - 1) / FPW;
-    const long long per_pass = (long long)gridDim.x * W;
-    const long long first = (long long)blockIdx.x * W;
-    const int n_pass = first < n_groups ? (int)((n_groups - first + per_pass - 1) / per_pass) : 0;
-    const uint32_t spp = (uint32_t)fp.n_chunks / kCPS;        // stages per pass (the stream is padded to whole stages)
-    if (!PRIV && wid == W) {                                  // ---- producer warp
-#ifndef PB_HOST_EMU
-        if (fp.no_tma == 3) {
-            const char *src = reinterpret_cast<const char *>(fp.stream);
-            uint32_t i = 0;
-            for (int p = 0; p < n_pass; ++p)
-                for (uint32_t s = 0; s < spp; ++s, ++i) {
-                    const uint32_t st = i & (kStages - 1);
-                    if (elect_one()) {
-                        mbar_wait(bars + (kStages + st) * 8u, ((i / kStages) & 1u) ^ 1u);
-                        bulk_load_cta(ring0 + st * kStageBytes, src + (size_t)s * kStageBytes, kStageBytes, bars + st * 8u);
-                    }
-                    __syncwarp();
-                }
-            return;
-        }
-#endif
-        if (fp.no_tma) {
-            const uint4 *src = reinterpret_cast<const uint4 *>(fp.stream);
-            uint4 *ring4 = reinterpret_cast<uint4 *>(RINGB);
-            uint32_t i = 0;
-            for (int p = 0; p < n_pass; ++p)
-                for (uint32_t s = 0; s < spp; ++s, ++i) {
-                    const uint32_t st = i & (kStages - 1);
-                    mbar_wait(bars + (kStages + st) * 8u, ((i / kStages) & 1u) ^ 1u);
-                    for (int k = lane; k < (int)(kStageBytes / 16); k += 32) ring4[st * (kStageBytes / 16) + k] = __ldg(src + (size_t)s * (kStageBytes / 16) + k);
-                    __threadfence_block();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(bars + st * 8u);
-                }
-            return;
-        }
-        // TMA producer.  The WHOLE warp stays in the loop and lane 0 issues: with lanes 1..31 retired and lane 0 left alone
-        // to wait and issue, the L = 1 kernels stopped (or faulted) as soon as an SM held its full complement of CTAs --
-        // measured on B200, round 2 (profiles/r2/README.md).  This form runs those shapes but still stops under CTA turnover
-        // (back-to-back one-wave launches on two streams); only the copy loop of a full warp (POLAR_B200_NO_TMA=1) runs
-        // everything.  Hence the private ring is the default.
-        {
-            const char *src = reinterpret_cast<const char *>(fp.stream);
-            uint32_t i = 0;
-            for (int p = 0; p < n_pass; ++p)
-                for (uint32_t s = 0; s < spp; ++s, ++i) {
-                    const uint32_t st = i & (kStages - 1);
-                    if (lane == 0) {
-                        mbar_wait(bars + (kStages + st) * 8u, ((i / kStages) & 1u) ^ 1u);     // slot free (passes at once the first time round)
-                        bulk_load(ring0 + st * kStageBytes, src + (size_t)s * kStageBytes, kStageBytes, bars + st * 8u);
-                    }
-                    __syncwarp();
-                }
-        }
-        return;
-    }
 
     uint32_t *V = sm + (size_t)wid * fp.warp_words;    // value levels gl+1..top, [word][lane]
     uint32_t *X = V + fp.vwords * 32;                  // partial sums, in place, [word][lane]
@@ -325,7 +187,7 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
     double *R1S = reinterpret_cast<double *>(SEL + 32);                  // [7][32] smallest |llr| of an R1 node (Fast kinds)
     uint32_t *R1Q = reinterpret_cast<uint32_t *>(R1S + 7 * 32);          // [7][32] their positions
     unsigned short *R1P = reinterpret_cast<unsigned short *>(R1S);       // [32][32] packed sort keys of an R1 node (dead before R1S/R1Q are written)
-    // workspace: kWsHeadWords of launch state (word 0 = next frame group, PRIV kernels), then one region per resident warp
+    // workspace: kWsHeadWords of launch state (word 0 = next frame group), then one region per resident warp
     uint32_t *G = ws + kWsHeadWords + ((size_t)blockIdx.x * W + wid) * fp.gwords * 32;  // value levels 1..gl, [word][lane], L2-resident
 
     LineState ls;
@@ -333,46 +195,18 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
     const smaddr_t ring_lane = ring0 + (unsigned)lane * 16u;   // this lane's 16 bytes of slot 0
     const char *stream_lane = reinterpret_cast<const char *>(fp.stream) + lane * 16;
     const uint32_t stream_bytes = (uint32_t)fp.n_chunks * 512u;
-    if (PRIV)
-        for (int i = 0; i < kPrivChunks - 1; ++i) { cp_async16(ring_lane + i * 512u, stream_lane + ls.fetch); ls.fetch += 512u; if (ls.fetch == stream_bytes) ls.fetch = 0u; }
+    for (int i = 0; i < kRingChunks - 1; ++i) { cp_async16(ring_lane + i * 512u, stream_lane + ls.fetch); ls.fetch += 512u; if (ls.fetch == stream_bytes) ls.fetch = 0u; }
     // the Fast-SSC variant has ~40 consumption sites: there the stream accessors are real (out-of-line) functions so
     // that the hot code stays inside the instruction cache; the plain variant inlines them
     auto next_chunk = [&]() -> uint4 {
-        if (PRIV) {
-            if (FAST && L > 1) {
-                const uint4 v = priv_fetch_outlined(ls.cc, ls.fetch, ring_lane, stream_lane);
-                ++ls.cc;
-                ls.fetch += 512u;
-                if (ls.fetch == stream_bytes) ls.fetch = 0u;
-                return v;
-            }
-            return priv_next_chunk(ls.cc, ls.fetch, ring_lane, stream_lane, stream_bytes);
-        }
-#ifdef PB_RING_VERIFY
-        if (fp.no_tma == 2) {   // debug build only: check every chunk read from the ring against the stream in global memory
-            const uint32_t c0 = ls.cc;
-            uint4 v = ring_next_chunk(ls.cc, ring_lane, bars, lane);
-            const uint32_t nch = (uint32_t)fp.n_chunks, k = c0 % nch;
-            const uint4 *gs = reinterpret_cast<const uint4 *>(fp.stream);
-            const uint4 e = __ldg(gs + (size_t)k * 32 + lane);
-            if (v.x != e.x || v.y != e.y || v.z != e.z || v.w != e.w) {
-                const uint4 prev = __ldg(gs + (size_t)((k + nch - kRingSlots % nch) % nch) * 32 + lane);
-                const uint4 nxt = __ldg(gs + (size_t)((k + kRingSlots) % nch) * 32 + lane);
-                int code = 0x40000000;
-                if (v.x == prev.x && v.y == prev.y && v.z == prev.z && v.w == prev.w) code |= 0x20000000;   // stale: the previous round's chunk
-                if (v.x == nxt.x && v.y == nxt.y && v.z == nxt.z && v.w == nxt.w) code |= 0x10000000;       // overwritten early: the next round's chunk
-                atomicOr(err_flag, code | (int)(c0 & 0xffffu) | ((wid & 7) << 16) | ((lane & 31) << 19));
-                v = e;
-            }
-            return v;
-        }
-#endif
         if (FAST && L > 1) {
-            const uint4 v = ring_fetch_outlined(ls.cc, ring_lane, bars, lane);
+            const uint4 v = ring_fetch_outlined(ls.cc, ls.fetch, ring_lane, stream_lane);
             ++ls.cc;
+            ls.fetch += 512u;
+            if (ls.fetch == stream_bytes) ls.fetch = 0u;
             return v;
         }
-        return ring_next_chunk(ls.cc, ring_lane, bars, lane);
+        return ring_next_chunk(ls.cc, ls.fetch, ring_lane, stream_lane, stream_bytes);
     };
     // upper-level steps and special nodes take their lines one at a time out of the current chunk.  In the Fast-SSC
     // variant `cur` is a queue with the next line in .x (no selects at the many call sites)
@@ -424,28 +258,13 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
     };
     auto nib = [](uint32_t w, int k) -> uint32_t { return (w >> (4 * k)) & 15u; };
 
-    for (int pass = 0; PRIV || pass < n_pass; ++pass) {
-        // PRIV kernels: the warps take their frame groups from a counter (zeroed by the host before the launch), so a warp
-        // that runs ahead -- they do, by a few per cent -- takes more of them and the launch ends without a tail.  The
-        // shared-ring kernels keep the static schedule (all warps of a CTA must consume the same number of passes).
-        long long g;
-        if (PRIV) {
-            unsigned t = 0;
-            if (lane == 0) t = atomicAdd(ws, 1u);
-            g = (long long)__shfl_sync(kFull, t, 0);
-            if (g >= n_groups) break;
-        } else {
-            g = ((long long)pass * gridDim.x + blockIdx.x) * W + wid;
-        }
-        if (g >= n_groups) {   // no group left for this warp: hand the pass's stages straight back
-            for (uint32_t s2 = 0; s2 < spp; ++s2, ls.cc += kCPS) {
-                const uint32_t st = (ls.cc & (kRingSlots - 1)) / kCPS;
-                mbar_wait(bars + st * 8u, (ls.cc / kRingSlots) & 1u);
-                __syncwarp();
-                if (lane == 0) mbar_arrive(bars + (kStages + st) * 8u);
-            }
-            continue;
-        }
+    for (;;) {
+        // the warps take their frame groups from a counter (zeroed by the host before the launch), so a warp that runs
+        // ahead -- they do, by a few per cent -- takes more of them and the launch ends without a tail
+        unsigned t = 0;
+        if (lane == 0) t = atomicAdd(ws, 1u);
+        const long long g = (long long)__shfl_sync(kFull, t, 0);
+        if (g >= n_groups) break;
         const uint32_t cc_pass = ls.cc;
         long long my_frame = g * FPW + grp;
         if (my_frame >= B) my_frame = B - 1;
@@ -720,13 +539,12 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
             if (!(L == 1 && spt == 0) && !(L > 1 && spt == 1)) ls.q = 4;
             uint4 ech = make_uint4(0, 0, 0, 0);
             auto elem_line = [&](int j) -> uint32_t {
-                if (PB_EXP_LINE) return next_line();
                 if ((j & 3) == 0) ech = next_chunk();
                 return (j & 3) == 0 ? ech.x : (j & 3) == 1 ? ech.y : (j & 3) == 2 ? ech.z : ech.w;
             };
             // a node of 2 elements leaves half a chunk: the following ops' lines continue there
             auto elem_done = [&]() {
-                if (PB_EXP_LINE || (temp & 3) == 0) return;
+                if ((temp & 3) == 0) return;
                 ls.q = 2;                                                  // temp == 2
                 if (FAST && L > 1) { ls.cur.x = ech.z; ls.cur.y = ech.w; }  // queue form: next line in .x
                 else ls.cur = ech;
@@ -1138,20 +956,14 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
             }
         }
         __syncwarp();
-        // hand back a partly consumed last stage; the next pass starts on the next stage
-        if (PRIV) {
-            while (ls.cc - cc_pass != spp * kCPS) (void)next_chunk();      // (the stream is padded to whole stages)
-        } else if (ls.cc & (kCPS - 1)) {
-            if (lane == 0) mbar_arrive(bars + (kStages + (ls.cc & (kRingSlots - 1)) / kCPS) * 8u);
-            ls.cc = (ls.cc + kCPS - 1) & ~(uint32_t)(kCPS - 1);
-        }
 #ifdef PB_HOST_EMU
-        if (ls.cc - cc_pass != spp * kCPS) { fprintf(stderr, "scl_lut_warp: pass consumed %u chunks, stream has %u\n", ls.cc - cc_pass, spp * kCPS); abort(); }
-#else
-        (void)cc_pass;
+        if (ls.cc - cc_pass > (uint32_t)fp.n_chunks) { fprintf(stderr, "scl_lut_warp: pass consumed %u chunks, stream has %d\n", ls.cc - cc_pass, fp.n_chunks); abort(); }
 #endif
+        // consume the rest of the pass's stream (its zero padding at the end), so that the next pass starts with chunk 0
+        // (n_chunks is a multiple of kRingChunks; the rounded bound makes 8 instructions less code in the Fast-SSC kernels)
+        while (ls.cc - cc_pass != (uint32_t)fp.n_chunks / kRingChunks * kRingChunks) (void)next_chunk();
     }
-    if (PRIV) cp_async_wait<0>();
+    cp_async_wait<0>();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1174,12 +986,12 @@ inline bool fast_upload(FastPlan *pl, const std::vector<T> &h, const T **out) {
 
 // Kernel instantiations live in their own translation units (pb_kernels.cu, compiled in parallel); the host side only
 // sees the dispatcher.
-const void *fast_kernel_fn(int logL, bool ca, bool fast, bool priv);
+const void *fast_kernel_fn(int logL, bool ca, bool fast);
 #ifdef PB_TU_SCL
-template <int LOGL, bool FAST, bool PRIV>
+template <int LOGL, bool FAST>
 inline const void *fast_kernel_fn_l(bool ca) {
-    if (LOGL == 0 || !ca) return PB_KFN(scl_lut_warp_kernel<LOGL, false, FAST, PRIV>);
-    return PB_KFN(scl_lut_warp_kernel<LOGL, (LOGL > 0), FAST, PRIV>);
+    if (LOGL == 0 || !ca) return PB_KFN(scl_lut_warp_kernel<LOGL, false, FAST>);
+    return PB_KFN(scl_lut_warp_kernel<LOGL, (LOGL > 0), FAST>);
 }
 #endif
 
@@ -1373,8 +1185,8 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
             while ((stream.size() / 32) % 4) stream.insert(stream.end(), 32, 0u);
         stream.insert(stream.end(), op_lines[i].begin(), op_lines[i].end());
     }
-    // pad to whole ring stages (kCPS chunks of 4 lines) and transpose each chunk to [lane][4]
-    while ((stream.size() / 32) % (4 * kCPS)) stream.insert(stream.end(), 32, 0u);
+    // pad to a multiple of kRingChunks chunks of 4 lines and transpose each chunk to [lane][4]
+    while ((stream.size() / 32) % (4 * kRingChunks)) stream.insert(stream.end(), 32, 0u);
     const int n_lines = (int)(stream.size() / 32);
     {
         std::vector<uint32_t> tr(stream.size());
@@ -1445,16 +1257,9 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
     pl->logL = logL;
     pl->ca = d.ca != 0;
     pl->fastk = max_special >= 0;
-    // Table ring: CTA-shared, filled by a producer warp with TMA bulk copies, or (POLAR_B200_RING=private) one private
-    // cp.async ring per warp
-    const char *ring_env = getenv("POLAR_B200_RING");
-    const bool priv = ring_env ? (ring_env[0] == 'p' || ring_env[0] == 'P') : PB_DEFAULT_RING_PRIVATE;
-    P.priv = priv ? 1 : 0;
-    const void *fn = fast_kernel_fn(logL, pl->ca, pl->fastk, priv);
-    // CTA shape: as many consumer warps per CTA as keep the SM's warp slots full (the ring and the producer warp are
-    // shared by the CTA); POLAR_B200_WARPS_PER_CTA overrides (tuning knob)
-    const size_t ring_shared = (size_t)kRingSlots * 512 + 2 * kStages * 8, ring_priv = (size_t)kPrivChunks * 512;
-    auto smem_for = [&](int w) { return (size_t)w * P.warp_words * 4 + (priv ? (size_t)w * ring_priv : ring_shared); };
+    const void *fn = fast_kernel_fn(logL, pl->ca, pl->fastk);
+    // CTA shape: as many warps per CTA as keep the SM's warp slots full; POLAR_B200_WARPS_PER_CTA overrides (tuning knob)
+    auto smem_for = [&](int w) { return (size_t)w * (P.warp_words * 4 + (size_t)kRingChunks * 512); };
     int best_w = 0, best_occ = 0, best_score = 0;
     const int warp_cap = (pl->fastk && L > 1 && !getenv("POLAR_B200_CTAS_PER_SM")) ? 12 : 1 << 20;   // resident warps per SM wanted at most
     const int want_w = getenv("POLAR_B200_WARPS_PER_CTA") ? atoi(getenv("POLAR_B200_WARPS_PER_CTA")) : 0;
@@ -1464,7 +1269,7 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
         const size_t smem = smem_for(w);
         if (smem > 200 * 1024) continue;
         int occ = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, (w + (priv ? 0 : 1)) * 32, smem) != cudaSuccess) { cudaGetLastError(); continue; }
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, w * 32, smem) != cudaSuccess) { cudaGetLastError(); continue; }
         // The Fast-SSC list variants are bound by instruction fetch (65 KB of code, 39 % of the stall samples "no
         // instruction"): every extra resident warp adds misses.  Measured on N=1024, L=8 (profiles/r2/README.md): 8 warps per
         // SM 9.1e6 frames/s, 12: 8.9e6, 16: 8.6e6, 21 (all that fit): 7.7e6.  They get 12 warps, in CTAs of 4 when those fit.
@@ -1475,7 +1280,6 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
     if (best_w < 1 || best_occ < 1) { free_fast_plan(pl); return; }
     P.warps = best_w;
     P.dbg = getenv("POLAR_B200_KDEBUG") ? atoi(getenv("POLAR_B200_KDEBUG")) : 0;
-    P.no_tma = getenv("POLAR_B200_NO_TMA") ? atoi(getenv("POLAR_B200_NO_TMA")) : 0;
     if (const char *e = getenv("POLAR_B200_CTAS_PER_SM")) best_occ = std::max(1, std::min(best_occ, atoi(e)));   // tuning / debug knob
     pl->smem = smem_for(best_w);
     pl->ws_bytes_per_cta = (size_t)P.gwords * 32 * 4 * best_w;
@@ -1496,11 +1300,9 @@ inline int launch_fast_lut(const Dev &d, const FastPlan &pl, const void *d_in, i
     const int grid = fast_grid(pl, B, sm_count);
     void *args[] = {(void *)&d, (void *)&pl.p, (void *)&d_in, (void *)&dtype, (void *)&d_out, (void *)&B, (void *)&ws,
                     (void *)&d_err, (void *)&dbg_pm, (void *)&dbg_win};
-    if (pl.p.priv) {      // the group counter of the dynamic schedule
-        cudaError_t e0 = cudaMemsetAsync(ws, 0, kWsHeadWords * 4, s);
-        if (e0 != cudaSuccess) return (int)e0;
-    }
-    cudaError_t e = cudaLaunchKernel(fast_kernel_fn(pl.logL, pl.ca, pl.fastk, pl.p.priv != 0), dim3(grid), dim3((pl.p.warps + (pl.p.priv ? 0 : 1)) * 32), args, pl.smem, s);
+    cudaError_t e0 = cudaMemsetAsync(ws, 0, kWsHeadWords * 4, s);   // the group counter of the dynamic schedule
+    if (e0 != cudaSuccess) return (int)e0;
+    cudaError_t e = cudaLaunchKernel(fast_kernel_fn(pl.logL, pl.ca, pl.fastk), dim3(grid), dim3(pl.p.warps * 32), args, pl.smem, s);
     if (e != cudaSuccess) return (int)e;
     return (int)cudaGetLastError();
 }

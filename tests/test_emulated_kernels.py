@@ -1,7 +1,7 @@
-"""The CUDA kernel SOURCE, compiled for the host by tools/emu (warps as fibers, shuffles / mbarriers / async copies
-emulated; test tooling like oracle/, never loaded by the package) and checked against the oracle: lets the GPU-less
-`-m "not gpu"` run exercise the kernels' logic -- op-list compiler, table stream and both ring protocols, dynamic group
-schedule, sorted-keeps fork, staging pipeline, multi-device dealing -- bit for bit.  The GPU tests remain the parity proof."""
+"""The CUDA kernel SOURCE, compiled for the host by tools/emu (warps as fibers, shuffles / async copies emulated; test
+tooling like oracle/, never loaded by the package) and checked against the oracle: lets the GPU-less `-m "not gpu"` run
+exercise the kernels' logic -- op-list compiler, table stream and ring, dynamic group schedule, sorted-keeps fork, staging
+pipeline, multi-device dealing -- bit for bit.  The GPU tests remain the parity proof."""
 import os
 import subprocess
 import sys
@@ -18,11 +18,8 @@ def emu_built():
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
 
 
-def _check(flt, env=None):
-    e = dict(os.environ)
-    e.pop("POLAR_B200_RING", None)
-    e.update(env or {})
-    r = subprocess.run([sys.executable, os.path.join(EMU, "check.py"), flt], capture_output=True, text=True, timeout=900, env=e)
+def _check(flt):
+    r = subprocess.run([sys.executable, os.path.join(EMU, "check.py"), flt], capture_output=True, text=True, timeout=900)
     assert r.returncode == 0 and r.stdout.strip().endswith("OK"), r.stdout[-3000:] + r.stderr[-2000:]
     assert "mismatching=   0" in r.stdout
     return r.stdout
@@ -32,8 +29,3 @@ def test_every_kernel_family_matches_the_oracle_under_the_emulator(emu_built):
     out = _check("")
     assert out.count("kernel=scl_lut_warp") >= 15 and "kernel=path_warp" in out
 
-
-def test_shared_ring_protocol_under_the_emulator(emu_built):
-    """the CTA-shared ring: producer / consumer hand-over through full / empty barriers, static schedule"""
-    for flt in ("ns_", "scl_l", "multi_pass", "cafast"):
-        _check(flt, {"POLAR_B200_RING": "shared"})

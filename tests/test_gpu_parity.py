@@ -348,9 +348,9 @@ def test_large_decoder_survives_a_smaller_one_created_later(monkeypatch, kind, f
 @pytest.mark.parametrize("kind,N,K,L,B", [("SCLUTDecoder", 256, 128, 1, 1 << 19), ("SCLUTDecoder", 1024, 512, 1, 113664 + 32),
                                            ("FastSCLUTDecoder", 1024, 512, 1, 1 << 17), ("SCLLUTDecoder", 512, 256, 4, 1 << 17)])
 def test_full_residency_batches(q, kind, N, K, L, B):
-    """Batches that fill every SM with its full complement of CTAs (and a few passes more).  Round 2 found the L = 1 kernels
-    hanging exactly there while every small-batch test passed (consumer warps suspended in mbarrier.try_wait on a barrier
-    completed by a TMA transaction; they poll with test_wait now)."""
+    """Batches that fill every SM with its full complement of CTAs (and a few passes more): resident CTAs at the
+    occupancy limit, warps taking several frame groups each, and the decoded copies of the same frames agreeing from the
+    first pass to the last -- shapes that no small-batch test reaches."""
     import torch
     from quantized_decoder_polar_codes_b200 import capi
     kw, x, _ = common.make_case(kind, N=N, K=K, L=L, B=2048, seed=9, tables="minsum", ebn0_db=3.0)

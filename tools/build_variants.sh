@@ -1,19 +1,21 @@
 #!/bin/bash
 # Library variants for same-box A/B runs of compile-time switches: tools/build_variants.sh "name:-DFLAG=.. -DFLAG2=.." ...
-# (only the L=8 private-ring objects k11 / k12 are rebuilt per variant); results in gpu_variants/libpolar_b200_<name>.so
+# (only the L=8 objects k1 / k2 are rebuilt per variant); results in gpu_variants/libpolar_b200_<name>.so
 set -e
-cd /root/repo/quantized_decoder_polar_codes_b200
+ROOT=$(cd "$(dirname "$0")/.." && pwd)
+OUT=$ROOT/gpu_variants
+cd "$ROOT/quantized_decoder_polar_codes_b200"
 F="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -fmad=false -Xcompiler -fPIC"
-mkdir -p /root/repo/gpu_variants
-OBJS=$(ls build/*.o | grep -v "_v_\|/k11.o\|/k12.o")
+mkdir -p "$OUT"
+OBJS=$(ls build/*.o | grep -v "_v_\|/k1.o\|/k2.o")
 for spec in "$@"; do
   name=${spec%%:*}; flags=${spec#*:}
-  nvcc $F -DPB_TU=11 $flags -c csrc/pb_kernels.cu -o build/k11_v_$name.o &
-  nvcc $F -DPB_TU=12 $flags -c csrc/pb_kernels.cu -o build/k12_v_$name.o &
+  nvcc $F -DPB_TU=1 $flags -c csrc/pb_kernels.cu -o build/k1_v_$name.o &
+  nvcc $F -DPB_TU=2 $flags -c csrc/pb_kernels.cu -o build/k2_v_$name.o &
 done
 wait
 for spec in "$@"; do
   name=${spec%%:*}
-  nvcc -shared -gencode arch=compute_100a,code=sm_100a -o /root/repo/gpu_variants/libpolar_b200_$name.so $OBJS build/k11_v_$name.o build/k12_v_$name.o
+  nvcc -shared -gencode arch=compute_100a,code=sm_100a -o "$OUT/libpolar_b200_$name.so" $OBJS build/k1_v_$name.o build/k2_v_$name.o
 done
-ls -la /root/repo/gpu_variants
+ls -la "$OUT"

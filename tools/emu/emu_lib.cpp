@@ -107,16 +107,13 @@ void launch(const std::function<void()> &body, dim3 grid, dim3 block, size_t sme
 #include "pb_capi.cu"
 
 namespace pb {
-#define PB_EMU_SCL(SUF, PRIV) \
-const void *scl_fn_l3_plain##SUF(bool ca) { return fast_kernel_fn_l<3, false, PRIV>(ca); } \
-const void *scl_fn_l3_fast##SUF(bool ca) { return fast_kernel_fn_l<3, true, PRIV>(ca); } \
-const void *scl_fn_l01##SUF(int logL, bool ca, bool fast) { \
-    if (logL == 0) return fast ? fast_kernel_fn_l<0, true, PRIV>(false) : fast_kernel_fn_l<0, false, PRIV>(false); \
-    return fast ? fast_kernel_fn_l<1, true, PRIV>(ca) : fast_kernel_fn_l<1, false, PRIV>(ca); \
-} \
-const void *scl_fn_l2##SUF(bool ca, bool fast) { return fast ? fast_kernel_fn_l<2, true, PRIV>(ca) : fast_kernel_fn_l<2, false, PRIV>(ca); }
-PB_EMU_SCL(, false)
-PB_EMU_SCL(_priv, true)
+const void *scl_fn_l3_plain(bool ca) { return fast_kernel_fn_l<3, false>(ca); }
+const void *scl_fn_l3_fast(bool ca) { return fast_kernel_fn_l<3, true>(ca); }
+const void *scl_fn_l01(int logL, bool ca, bool fast) {
+    if (logL == 0) return fast ? fast_kernel_fn_l<0, true>(false) : fast_kernel_fn_l<0, false>(false);
+    return fast ? fast_kernel_fn_l<1, true>(ca) : fast_kernel_fn_l<1, false>(ca);
+}
+const void *scl_fn_l2(bool ca, bool fast) { return fast ? fast_kernel_fn_l<2, true>(ca) : fast_kernel_fn_l<2, false>(ca); }
 const void *path_fn_lut(int logL) { return path_kernel_fn_d<DOM_LUT>(logL); }
 const void *path_fn_float(int logL) { return path_kernel_fn_d<DOM_FLOAT>(logL); }
 const void *path_fn_uniform(int logL) { return path_kernel_fn_d<DOM_UNIFORM>(logL); }
