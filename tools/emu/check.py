@@ -55,6 +55,9 @@ CASES = [
     ("fastsc_1024", "FastSCLUTDecoder", dict(N=1024, K=512, B=100, tables="minsum")),
     ("float_scl", "SCLDecoder", dict(N=128, K=64, L=8, B=16, tables="channel")),
     ("uniform_l32", "SCLUniformQuantizedDecoder", dict(N=128, K=64, L=32, B=8)),
+    # N=32: the depth top-1 node of SUB16 is at depth 1, right below the root
+    ("sclut_32", "SCLUTDecoder", dict(N=32, K=16, B=200)),
+    ("scl_32", "SCLLUTDecoder", dict(N=32, K=16, L=8, B=40)),
 ]
 
 

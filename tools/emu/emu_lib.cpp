@@ -132,6 +132,17 @@ const void *generic_kernel_fn(int dom, bool l, bool w) {
 }
 }  // namespace pb
 
+// The compiled scl_lut_warp walk of a decoder (the `_handle` of a pybind decoder): hist[type * 32 + depth] = number of
+// ops of that type at that depth (types < 16), plus n_ops and n_chunks.  Returns -1 when the decoder is not on scl_lut_warp.
+extern "C" int pb_emu_fast_plan(const pd_decoder *dec, int *hist, int *n_ops, int *n_chunks) {
+    if (!dec->fast.ok) return -1;
+    memset(hist, 0, 16 * 32 * sizeof(int));
+    for (const uint2 &o : dec->fast.ops) hist[(o.x & 15u) * 32 + ((o.x >> 8) & 31u)]++;
+    *n_ops = dec->fast.p.n_ops;
+    *n_chunks = dec->fast.p.n_chunks;
+    return 0;
+}
+
 // entry points of the real library that the emulator does not provide (the pybind module links them)
 extern "C" {
 int pd_count_errors(const uint8_t *, const uint8_t *, int64_t, int32_t, unsigned long long *, void *) { return PD_ECUDA; }
