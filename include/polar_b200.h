@@ -156,6 +156,7 @@ int pd_count_errors(const uint8_t *dev_decoded, const uint8_t *dev_truth, int64_
  * (mainQuantizedDecoder_LLRDomain.py:151-176): random message -> [CRC] -> polar encode (natural order) ->
  * BPSK + AWGN(sigma) -> llr = 2y/sigma^2 -> channel quantizer (edges + lut, the driver's bisect rule), all on
  * the GPU (Philox counter RNG: frame i of a run always sees the same noise whatever the batch split / GPU).
+ * pd_sim_set_channel switches to the front ends of the probability-domain and continuous-domain drivers.
  * Decode with pd_decode_device and count with pd_count_errors afterwards. */
 typedef struct pd_sim pd_sim;
 typedef struct pd_sim_config {
@@ -172,10 +173,41 @@ typedef struct pd_sim_config {
 } pd_sim_config;
 int pd_sim_create(const pd_sim_config *cfg, pd_sim **out);
 void pd_sim_destroy(pd_sim *sim);
-/* Generates frames [first_frame, first_frame+B) of the run `seed`: dev_msg [B][A] uint8 message bits,
- * dev_out [B][N] uint8 symbols (quantizer given) or fp64 LLRs.  Asynchronous on cuda_stream. */
+/* Generates frames [first_frame, first_frame+B) of the run `seed`: dev_msg [B][A] uint8 message bits and
+ * dev_out [B][N] in the type of the current channel mode (see pd_sim_set_channel): uint8 symbols for PD_SIM_LLR_QUANT
+ * and PD_SIM_Y_QUANT, fp64 for PD_SIM_LLR and PD_SIM_LLR_UNIFORM.  Frame i of a run has the same message and the same
+ * channel output y in every mode.  Asynchronous on cuda_stream. */
 int pd_sim_generate(pd_sim *sim, double sigma, int64_t B, uint64_t seed, uint64_t first_frame,
                     uint8_t *dev_msg, void *dev_out, void *cuda_stream);
+
+/* Channel front end of a pd_sim: what pd_sim_generate stores for each code bit, from y = 1-2x + sigma*n and
+ * llr = 2y/sigma^2.  One mode per reference driver. */
+#define PD_SIM_LLR 0          /* fp64 LLRs                                   (what pd_sim_create sets without edges) */
+#define PD_SIM_LLR_QUANT 1    /* LLR-domain driver: edges + chan_lut -> uint8 (what pd_sim_create sets with edges)    */
+#define PD_SIM_Y_QUANT 2      /* probability-domain driver: y cut at edges[q_channel+1] -> uint8                      */
+#define PD_SIM_LLR_UNIFORM 3  /* continuous-domain driver: QUniform(llr, v, r) -> fp64                               */
+typedef struct pd_sim_channel {
+    int32_t mode;
+    const double *edges; int32_t n_edges;   /* LLR_QUANT, Y_QUANT */
+    const uint8_t *chan_lut;                /* LLR_QUANT: [n_edges-1] */
+    int32_t q_channel;                      /* LLR_QUANT, Y_QUANT */
+    double r; int32_t v;                    /* LLR_UNIFORM: step and level count */
+} pd_sim_channel;
+/* Replaces the channel front end of `sim`; the code, CRC and device stay.  A sweep over Eb/N0 calls this once per point,
+ * as the drivers design a new channel quantizer at every point.
+ *   PD_SIM_LLR          nothing else is read.
+ *   PD_SIM_LLR_QUANT    symbol = 0 if llr <= edges[0], q_channel-1 if llr >= edges[n_edges-1],
+ *                       else chan_lut[bisect_left(edges[0..n_edges-2], llr) - 1]  (mainQuantizedDecoder_LLRDomain.py:167-176).
+ *                       n_edges >= 2, chan_lut entries < q_channel.
+ *   PD_SIM_Y_QUANT      symbol = 0 if y <= edges[0], q_channel-1 if y >= edges[q_channel],
+ *                       else bisect_left(edges, y) - 1  (mainQuantizedDecoder_ProbabilityDomain.py:153-177: the MMI channel
+ *                       quantizer's edges interval_x[channel_lut]).  n_edges == q_channel + 1.
+ *   PD_SIM_LLR_UNIFORM  QUniform (mainQuantizedDecoder_ContinuousDomain.py:29-32): with bound = (v/2 - 0.5) r,
+ *                       out = sign(llr) (bound - r/2) if |llr| > bound, else (floor(llr/r) + 0.5) r.  r > 0 finite, v >= 2.
+ * q_channel is in [1,256]; edges are ascending and not NaN.  Violations return PD_EINVAL and leave the sim unchanged.
+ * The tables are copied into new device buffers that live until pd_sim_destroy: a pd_sim_generate already enqueued on
+ * some stream keeps reading the tables it was launched with, so this call needs no synchronisation. */
+int pd_sim_set_channel(pd_sim *sim, const pd_sim_channel *ch);
 
 /* Blind-detection entry (kinds PD_BD_DMETRIC / PD_BD_CASCL; fp64 LLR input [B][N]).
  *   PD_BD_DMETRIC: out_metric[b] = DMetricCalculator.calculate(llr_b) (DMetric.cpp:25-176); out_bits / out_pass unused (may be NULL).

@@ -9,6 +9,7 @@ LIB_PATH = os.path.join(_HERE, "libpolar_b200.so")
 
 PD_U8, PD_I32, PD_F64 = 0, 1, 2
 PD_OK, PD_EINVAL, PD_ECUDA, PD_ERANGE, PD_ENOMEM = 0, 1, 2, 3, 4
+PD_SIM_LLR, PD_SIM_LLR_QUANT, PD_SIM_Y_QUANT, PD_SIM_LLR_UNIFORM = 0, 1, 2, 3      # pd_sim_channel.mode
 
 _lib = None
 
@@ -43,6 +44,7 @@ def lib():
         L.pd_sim_create.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
         L.pd_sim_destroy.argtypes = [C.c_void_p]
         L.pd_sim_generate.argtypes = [C.c_void_p, C.c_double, C.c_int64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.pd_sim_set_channel.argtypes = [C.c_void_p, C.c_void_p]
         L.pd_sim_encode.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]
         L.pd_sim_encode_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
         L.pd_decode_bd.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -92,3 +94,8 @@ class SimConfig(C.Structure):
     _fields_ = [("N", C.c_int32), ("K", C.c_int32), ("A", C.c_int32), ("device", C.c_int32),
                 ("frozen_bits", C.c_void_p), ("crc_n", C.c_int32), ("crc_loc", C.c_void_p), ("crc_loc_len", C.c_int32),
                 ("edges", C.c_void_p), ("n_edges", C.c_int32), ("chan_lut", C.c_void_p), ("q_channel", C.c_int32)]
+
+
+class SimChannel(C.Structure):
+    _fields_ = [("mode", C.c_int32), ("edges", C.c_void_p), ("n_edges", C.c_int32), ("chan_lut", C.c_void_p),
+                ("q_channel", C.c_int32), ("r", C.c_double), ("v", C.c_int32)]

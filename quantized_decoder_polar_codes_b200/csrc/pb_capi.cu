@@ -1160,6 +1160,16 @@ void pd_sim_destroy(pd_sim *S) {
     delete S;
 }
 
+// copies `bytes` host bytes into a new device buffer owned by S (freed by pd_sim_destroy)
+static int sim_upload(pd_sim *S, const void *h, size_t bytes, const void **dst) {
+    void *p = nullptr;
+    if (cudaMalloc(&p, std::max<size_t>(bytes, 16)) != cudaSuccess) return fail(PD_ECUDA, "cudaMalloc failed");
+    S->allocs.push_back(p);
+    if (bytes && cudaMemcpy(p, h, bytes, cudaMemcpyHostToDevice) != cudaSuccess) return fail(PD_ECUDA, "cudaMemcpy failed");
+    *dst = p;
+    return PD_OK;
+}
+
 int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
     if (!c || !out || !c->frozen_bits) return fail(PD_EINVAL, "null argument");
     *out = nullptr;
@@ -1179,16 +1189,8 @@ int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
     S->device = c->device;
     SimDev &d = S->dev;
     d.N = N; d.K = c->K; d.A = c->A; d.crc_n = c->crc_n;
-    auto up = [&](const void *h, size_t bytes, const void **dst) -> int {
-        void *p = nullptr;
-        if (cudaMalloc(&p, std::max<size_t>(bytes, 16)) != cudaSuccess) return fail(PD_ECUDA, "cudaMalloc failed");
-        S->allocs.push_back(p);
-        if (bytes && cudaMemcpy(p, h, bytes, cudaMemcpyHostToDevice) != cudaSuccess) return fail(PD_ECUDA, "cudaMemcpy failed");
-        *dst = p;
-        return PD_OK;
-    };
     int rc;
-    if ((rc = up(info_pos.data(), info_pos.size() * 4, (const void **)&d.info_pos))) { pd_sim_destroy(S); return rc; }
+    if ((rc = sim_upload(S, info_pos.data(), info_pos.size() * 4, (const void **)&d.info_pos))) { pd_sim_destroy(S); return rc; }
     std::vector<uint32_t> rem(c->A, 0);
     if (c->crc_n > 0) {
         std::vector<int> poly(c->crc_n + 1, 0);
@@ -1209,7 +1211,7 @@ int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
             rem[k] = reg;
         }
     }
-    if ((rc = up(rem.data(), rem.size() * 4, (const void **)&d.crc_rem))) { pd_sim_destroy(S); return rc; }
+    if ((rc = sim_upload(S, rem.data(), rem.size() * 4, (const void **)&d.crc_rem))) { pd_sim_destroy(S); return rc; }
     if (N <= 1024) {
         std::vector<EncWord> tab(32);
         memset(tab.data(), 0, tab.size() * sizeof(EncWord));
@@ -1222,15 +1224,58 @@ int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
             enc_expand_masks(m, tab[w].mv);
             before += (uint32_t)__builtin_popcount(m);
         }
-        if ((rc = up(tab.data(), tab.size() * sizeof(EncWord), (const void **)&S->enc_tab))) { pd_sim_destroy(S); return rc; }
+        if ((rc = sim_upload(S, tab.data(), tab.size() * sizeof(EncWord), (const void **)&S->enc_tab))) { pd_sim_destroy(S); return rc; }
     }
     if (c->edges) {
-        if ((rc = up(c->edges, (size_t)c->n_edges * 8, (const void **)&d.edges)) ||
-            (rc = up(c->chan_lut, (size_t)(c->n_edges - 1), (const void **)&d.chan_lut))) { pd_sim_destroy(S); return rc; }
+        if ((rc = sim_upload(S, c->edges, (size_t)c->n_edges * 8, (const void **)&d.edges)) ||
+            (rc = sim_upload(S, c->chan_lut, (size_t)(c->n_edges - 1), (const void **)&d.chan_lut))) { pd_sim_destroy(S); return rc; }
         d.n_edges = c->n_edges;
         d.q_channel = c->q_channel;
+        d.mode = PD_SIM_LLR_QUANT;
+    } else {
+        d.mode = PD_SIM_LLR;
     }
     *out = S;
+    return PD_OK;
+}
+
+int pd_sim_set_channel(pd_sim *S, const pd_sim_channel *ch) {
+    if (!S || !ch) return fail(PD_EINVAL, "null argument");
+    SimDev d = S->dev;
+    d.edges = nullptr; d.n_edges = 0; d.chan_lut = nullptr; d.q_channel = 0;
+    d.r = d.bound = d.sat = 0.0;
+    d.mode = ch->mode;
+    const bool llr_quant = ch->mode == PD_SIM_LLR_QUANT, y_quant = ch->mode == PD_SIM_Y_QUANT;
+    if (llr_quant || y_quant) {
+        if (!ch->edges) return fail(PD_EINVAL, "edges is NULL");
+        if (ch->n_edges < 2) return fail(PD_EINVAL, "n_edges=%d: need at least 2 edges", ch->n_edges);
+        if (ch->q_channel < 1 || ch->q_channel > 256) return fail(PD_EINVAL, "q_channel=%d must be in [1,256]", ch->q_channel);
+        for (int i = 0; i < ch->n_edges; ++i)
+            if (std::isnan(ch->edges[i]) || (i > 0 && !(ch->edges[i] >= ch->edges[i - 1])))
+                return fail(PD_EINVAL, "edges must be ascending and not NaN (edge %d)", i);
+        if (y_quant && ch->n_edges != ch->q_channel + 1)
+            return fail(PD_EINVAL, "PD_SIM_Y_QUANT needs n_edges == q_channel + 1 (got n_edges=%d, q_channel=%d)", ch->n_edges, ch->q_channel);
+        if (llr_quant) {
+            if (!ch->chan_lut) return fail(PD_EINVAL, "chan_lut is NULL");
+            for (int i = 0; i < ch->n_edges - 1; ++i)
+                if (ch->chan_lut[i] >= ch->q_channel) return fail(PD_EINVAL, "chan_lut[%d]=%d is not below q_channel=%d", i, ch->chan_lut[i], ch->q_channel);
+        }
+        d.n_edges = ch->n_edges;
+        d.q_channel = ch->q_channel;
+    } else if (ch->mode == PD_SIM_LLR_UNIFORM) {
+        if (!(ch->r > 0) || !std::isfinite(ch->r)) return fail(PD_EINVAL, "r=%g must be finite and > 0", ch->r);
+        if (ch->v < 2) return fail(PD_EINVAL, "v=%d must be >= 2", ch->v);
+        d.r = ch->r;
+        d.bound = ((double)(ch->v / 2) - 0.5) * ch->r;   // M = (v//2 - 0.5)*r and M - 0.5*r, numpy's operation order
+        d.sat = d.bound - 0.5 * ch->r;
+    } else if (ch->mode != PD_SIM_LLR) {
+        return fail(PD_EINVAL, "unknown channel mode %d", ch->mode);
+    }
+    CUDA_TRY(cudaSetDevice(S->device));
+    int rc;
+    if (d.n_edges && (rc = sim_upload(S, ch->edges, (size_t)d.n_edges * 8, (const void **)&d.edges))) return rc;
+    if (llr_quant && (rc = sim_upload(S, ch->chan_lut, (size_t)(d.n_edges - 1), (const void **)&d.chan_lut))) return rc;
+    S->dev = d;
     return PD_OK;
 }
 

@@ -2,7 +2,15 @@
 // quantizer, one warp per frame.  Mirrors the loop body of the reference drivers
 // (mainQuantizedDecoder_LLRDomain.py:151-176) and the encoder / CRC conventions of SURVEY.md 8(c):
 //   u[non-frozen] = msg || crc(msg),  x = u F^{(x)n} in natural order,  y = 1-2x + sigma*n,  llr = 2y/sigma^2,
-//   symbol = 0 if llr <= edges[0], Qc-1 if llr >= edges[M], else lut[bisect_left(edges[:-1], llr) - 1].
+// then stores, per SimDev::mode (the PD_SIM_* values of include/polar_b200.h), what the driver in question feeds its decoder:
+//   PD_SIM_LLR          llr (fp64)
+//   PD_SIM_LLR_QUANT    0 if llr <= edges[0], Qc-1 if llr >= edges[M], else lut[bisect_left(edges[:-1], llr) - 1]  (uint8;
+//                       LLR-domain driver, mainQuantizedDecoder_LLRDomain.py:167-176)
+//   PD_SIM_Y_QUANT      0 if y <= edges[0], Qc-1 if y >= edges[M], else bisect_left(edges, y) - 1  (uint8; M = Qc;
+//                       probability-domain driver, mainQuantizedDecoder_ProbabilityDomain.py:153-177)
+//   PD_SIM_LLR_UNIFORM  QUniform: copysign(sat, llr) if |llr| > bound, else (floor(llr/r) + 0.5) r  (fp64;
+//                       continuous-domain driver, mainQuantizedDecoder_ContinuousDomain.py:29-32)
+// The mode only picks the last step: message, code word and noise are the same in every mode.
 // Noise is Philox4x32-10 keyed by (seed, frame, lane): frame i sees the same noise however the run is split.
 #pragma once
 #include <cuda_runtime.h>
@@ -10,16 +18,20 @@
 
 #include <cstdint>
 
+#include "../../include/polar_b200.h"
+
 namespace pb {
 
 struct SimDev {
     int N, K, A, crc_n;
     const int32_t *info_pos;     // [K]
     const uint32_t *crc_rem;     // [A] remainder of unit message bit k (MSB-first long division), crc_n <= 32
-    const double *edges;         // [n_edges] or nullptr
+    const double *edges;         // [n_edges] (LLR_QUANT, Y_QUANT) or nullptr
     int n_edges;
-    const uint8_t *chan_lut;     // [n_edges-1]
+    const uint8_t *chan_lut;     // [n_edges-1] (LLR_QUANT)
     int q_channel;
+    int mode;                    // PD_SIM_*
+    double r, bound, sat;        // LLR_UNIFORM: step, saturation threshold and saturated value (computed on the host)
 };
 
 __global__ void __launch_bounds__(128)
@@ -91,22 +103,26 @@ sim_generate_kernel(const SimDev s, double sigma, long long B, unsigned long lon
                 const uint32_t xb = (U[p >> 5] >> (p & 31)) & 1u;
                 const double y = (1.0 - 2.0 * (double)xb) + sigma * (h ? nz.y : nz.x);
                 const double llr = y * inv;
-                if (s.edges == nullptr) {
-                    reinterpret_cast<double *>(out)[(size_t)f * N + p] = llr;
+                const size_t o = (size_t)f * N + p;
+                if (s.mode == PD_SIM_LLR) {
+                    reinterpret_cast<double *>(out)[o] = llr;
+                } else if (s.mode == PD_SIM_LLR_UNIFORM) {
+                    reinterpret_cast<double *>(out)[o] = fabs(llr) > s.bound ? copysign(s.sat, llr) : (floor(llr / s.r) + 0.5) * s.r;
                 } else {
+                    const double v = s.mode == PD_SIM_Y_QUANT ? y : llr;
                     int sym;
                     const int M = s.n_edges - 1;
-                    if (llr <= s.edges[0]) sym = 0;
-                    else if (llr >= s.edges[M]) sym = s.q_channel - 1;
-                    else {   // bisect_left(edges[0..M-1], llr) - 1
+                    if (v <= s.edges[0]) sym = 0;
+                    else if (v >= s.edges[M]) sym = s.q_channel - 1;
+                    else {   // bisect_left(edges[0..M-1], v); v < edges[M], so it is also bisect_left over all M+1 edges
                         int lo = 0, hi = M;
                         while (lo < hi) {
                             const int mid = (lo + hi) >> 1;
-                            if (s.edges[mid] < llr) lo = mid + 1; else hi = mid;
+                            if (s.edges[mid] < v) lo = mid + 1; else hi = mid;
                         }
-                        sym = s.chan_lut[lo - 1];
+                        sym = s.mode == PD_SIM_Y_QUANT ? lo - 1 : s.chan_lut[lo - 1];
                     }
-                    reinterpret_cast<uint8_t *>(out)[(size_t)f * N + p] = (uint8_t)sym;
+                    reinterpret_cast<uint8_t *>(out)[o] = (uint8_t)sym;
                 }
             }
         }

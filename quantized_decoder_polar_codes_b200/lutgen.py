@@ -295,3 +295,16 @@ def channel_llr_density_table(M, low, high, mu1, mu2, sigma):
         pyx[i] = np.sum(d) * delta
         quanta[i] = np.sum(x[sel] * d) / np.sum(d)
     return pyx, edges, quanta
+
+
+def llr_channel_quantizer(sigma, q_uniform=128, q_channel=16, device=0):
+    """The channel quantizer the LLR-domain driver builds for a noise level (mainQuantizedDecoder_LLRDomain.py:143-145):
+    q_uniform uniform LLR cells on [-E-3D, E+3D] (E = 2/sigma^2, D = sqrt(2E)) merged to q_channel symbols by the
+    minimum-distortion quantizer (LLRQuantizer.find_OptLS_quantizer, here optls_quantize_batch).  The counterpart of
+    mmi_channel_quantizer.  -> cell edges interval_x [q_uniform+1] float64, channel_lut [q_uniform] uint8: the arguments of
+    simulate.LLRQuantizer."""
+    E = 2 / sigma ** 2
+    D = np.sqrt(2 * E)
+    pyx, interval_x, quanta = channel_llr_density_table(q_uniform, -E - 3 * D, E + 3 * D, E, -E, D)
+    _, _, luts = optls_quantize_batch([pyx], [quanta], q_channel, device)
+    return interval_x, luts[0].astype(np.uint8)

@@ -3,10 +3,28 @@
 quantizer, decode, BER/BLER counters -- without ever leaving the device.  One process per GPU; with
 torch.distributed initialised the two counters are all-reduced (NCCL) at the end of each Eb/N0 point.
 
+The channel front end is one of the reference drivers' (csrc/pb_sim.cuh); `set_channel` swaps it between Eb/N0 points, which
+is how the drivers' outer loop runs (a new channel quantizer per point, same code and CRC):
+
+    # LLR-domain driver, MinDistortion tables: symbol = lut[bisect of the LLR over the uniform cells]
     sim = Simulator(decoder, frozen_bits, A=512, crc=False, channel_quantizer=(edges, lut, 16))
-    res = sim.run(ebn0_db=2.0, frames=1 << 22)        # {'ber':..., 'bler':..., 'frames':..., ...}
+    for eb in (1.0, 2.0, 3.0):
+        edges, lut = lutgen.llr_channel_quantizer(awgn_sigma(eb, 512 / 1024))
+        sim.set_channel(LLRQuantizer(edges, lut, 16))
+        res = sim.run(ebn0_db=eb, frames=1 << 22, max_block_errors=1000)    # {'ber':..., 'bler':..., 'frames':..., ...}
+
+    # probability-domain driver, MMI tables: y cut at the MMI channel quantizer's edges, symbol = cell index
+    _, interval_x, channel_lut = lutgen.mmi_channel_quantizer(sigma)
+    sim.set_channel(YQuantizer(interval_x[channel_lut], 16))
+
+    # continuous-domain driver, uniformly quantized decoders: QUniform of the LLR with the root step, fp64
+    r_f, r_g = simulation.uniform_quantizer_steps(N, 16, sigma)
+    sim.set_channel(UniformLLR(r_f[0], 16))
+
+`set_channel(None)` gives fp64 LLRs (the float decoders).
 """
 import ctypes as C
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -16,7 +34,36 @@ from . import distributed as D
 from .simulation import CRC24_LOC, awgn_sigma
 
 
+class LLRQuantizer(NamedTuple):
+    """LLR-domain driver (mainQuantizedDecoder_LLRDomain.py:167-176): 0 if llr <= edges[0], q_channel-1 if llr >= edges[-1],
+    else lut[bisect_left(edges[:-1], llr) - 1].  edges: interval_x [M+1], lut: channel_lut [M].  uint8 symbols."""
+    edges: np.ndarray
+    lut: np.ndarray
+    q_channel: int
+
+
+class YQuantizer(NamedTuple):
+    """Probability-domain driver (mainQuantizedDecoder_ProbabilityDomain.py:153-177): y (not the LLR) cut at the MMI channel
+    quantizer's edges interval_x[channel_lut] [q_channel+1]: 0 if y <= edges[0], q_channel-1 if y >= edges[-1], else
+    searchsorted(edges, y, 'left') - 1.  uint8 symbols."""
+    edges: np.ndarray
+    q_channel: int
+
+
+class UniformLLR(NamedTuple):
+    """Continuous-domain driver's QUniform (mainQuantizedDecoder_ContinuousDomain.py:29-32) with step r = decoder_r_f[0] and
+    v levels: M = (v//2 - 0.5) r, sign(llr) (M - r/2) if |llr| > M, else (floor(llr/r) + 0.5) r.  fp64."""
+    r: float
+    v: int
+
+
+def _ptr(a):
+    return None if a is None else a.ctypes.data
+
+
 class Simulator:
+    """channel_quantizer: None (fp64 LLRs), an (edges, lut, q_channel) tuple or LLRQuantizer, a YQuantizer or a UniformLLR."""
+
     def __init__(self, decoder, frozen_bits, A, crc=False, channel_quantizer=None, device=None, crc_n=24, crc_loc=CRC24_LOC):
         self.dec = decoder
         self.lib = capi.lib()
@@ -32,17 +79,58 @@ class Simulator:
         loc = np.ascontiguousarray(crc_loc, dtype=np.int32)
         if crc:
             cfg.crc_n, cfg.crc_loc, cfg.crc_loc_len = crc_n, loc.ctypes.data, loc.size
-        self.quantized = channel_quantizer is not None
-        if self.quantized:
+        later = None
+        if isinstance(channel_quantizer, (YQuantizer, UniformLLR)):     # front ends pd_sim_config has no fields for
+            later, channel_quantizer = channel_quantizer, None
+        self.channel = None
+        if channel_quantizer is not None:
             edges, lut, qc = channel_quantizer
             edges = np.ascontiguousarray(edges, dtype=np.float64)
             lut = np.ascontiguousarray(lut, dtype=np.uint8)
             assert lut.size == edges.size - 1
             cfg.edges, cfg.n_edges, cfg.chan_lut, cfg.q_channel = edges.ctypes.data, edges.size, lut.ctypes.data, int(qc)
+            self.channel = LLRQuantizer(edges, lut, int(qc))
         h = C.c_void_p()
         capi.check(self.lib.pd_sim_create(C.byref(cfg), C.byref(h)))
         self._h = h
         self.rate = self.A / self.N
+        if later is not None:
+            self.set_channel(later)
+
+    @property
+    def quantized(self):
+        """True when the channel front end emits uint8 symbols (LLRQuantizer, YQuantizer), False for fp64 output."""
+        return isinstance(self.channel, (LLRQuantizer, YQuantizer))
+
+    def set_channel(self, channel):
+        """Replaces the channel front end (pd_sim_set_channel): None, LLRQuantizer, YQuantizer or UniformLLR.  The code and CRC
+        stay; frames already enqueued by generate() keep the tables they were launched with.  Raises ValueError on a bad
+        quantizer."""
+        ch = capi.SimChannel()
+        edges = lut = None
+        if channel is None:
+            ch.mode = capi.PD_SIM_LLR
+        elif isinstance(channel, LLRQuantizer):
+            edges = None if channel.edges is None else np.ascontiguousarray(channel.edges, dtype=np.float64)
+            if channel.lut is not None:
+                lut = np.asarray(channel.lut)
+                if lut.size and (lut.min() < 0 or lut.max() > 255):
+                    raise ValueError("channel lut entries must be in [0,255]")
+                lut = np.ascontiguousarray(lut, dtype=np.uint8)
+                if edges is not None and lut.size != edges.size - 1:
+                    raise ValueError(f"the lut has {lut.size} entries for {edges.size} edges (need one per cell)")
+            ch.mode, ch.q_channel = capi.PD_SIM_LLR_QUANT, int(channel.q_channel)
+        elif isinstance(channel, YQuantizer):
+            edges = None if channel.edges is None else np.ascontiguousarray(channel.edges, dtype=np.float64)
+            ch.mode, ch.q_channel = capi.PD_SIM_Y_QUANT, int(channel.q_channel)
+        elif isinstance(channel, UniformLLR):
+            ch.mode, ch.r, ch.v = capi.PD_SIM_LLR_UNIFORM, float(channel.r), int(channel.v)
+        else:
+            raise TypeError(f"unknown channel front end {type(channel).__name__}")
+        ch.edges, ch.chan_lut = _ptr(edges), _ptr(lut)
+        ch.n_edges = 0 if edges is None else edges.size
+        capi.check(self.lib.pd_sim_set_channel(self._h, C.byref(ch)))
+        self.channel = channel
 
     def __del__(self):
         try:

@@ -149,6 +149,7 @@ int pd_count_errors(const uint8_t *, const uint8_t *, int64_t, int32_t, unsigned
 int pd_sim_create(const pd_sim_config *, pd_sim **) { return PD_ECUDA; }
 void pd_sim_destroy(pd_sim *) {}
 int pd_sim_generate(pd_sim *, double, int64_t, uint64_t, uint64_t, uint8_t *, void *, void *) { return PD_ECUDA; }
+int pd_sim_set_channel(pd_sim *, const pd_sim_channel *) { return PD_ECUDA; }
 int pd_sim_encode(pd_sim *, int, const uint8_t *, int64_t, uint8_t *) { return PD_ECUDA; }
 int pd_sim_encode_device(pd_sim *, int, const uint8_t *, int64_t, uint8_t *, void *) { return PD_ECUDA; }
 int pd_mmi_slice_sums(const double *, const double *, int32_t, int32_t, int32_t, double *, double *, int32_t) { return PD_ECUDA; }
