@@ -75,7 +75,8 @@ typedef enum pd_status {
  */
 typedef struct pd_config {
     int32_t kind;                 /* pd_kind */
-    int32_t N, K, A, L;           /* A: CA kinds only; L: list kinds only */
+    int32_t N, K, A, L;           /* A: CA kinds only; L: list kinds only, 1..32, or 64, 128, 256 with N >= 32 (those three
+                                     run on "path_cta"; PD_BD_CASCL takes 1..32 only).  Other values: PD_EINVAL */
     int32_t device;               /* CUDA device ordinal */
     const int32_t *frozen_bits;   /* [N], 1 = frozen (indicator mask, mainFPDecoder.py:49,58) */
     const int32_t *node_type;     /* [2N-1] Fast kinds: -1 ordinary, 0 R0, 1 R1, 2 REP, 3 SPC (IdentifyNodes.py) */
@@ -109,7 +110,7 @@ void pd_destroy(pd_decoder *dec);
 int pd_out_len(const pd_decoder *dec);
 int pd_code_len(const pd_decoder *dec);
 /* Frames that one full wave of the (persistent) decode kernel holds in flight on the decoder's GPU: SMs x resident warps x
- * frames per warp; 0 for the CTA-per-frame generic kernel.  The scl_lut_warp kernels hand frame groups to their warps from a
+ * frames per warp (path_cta, L >= 64: SMs x resident CTAs, one frame per CTA); 0 for the CTA-per-frame generic kernel.  The scl_lut_warp kernels hand frame groups to their warps from a
  * counter, so any batch size runs without a tail in one launch; the statically scheduled kernels (fp64 family, Fast-SSC
  * variants) get large batches as overlapping one-wave launches, and there a multiple of this number has no tail. */
 int64_t pd_wave_frames(const pd_decoder *dec, int in_dtype);
@@ -263,7 +264,8 @@ int pd_mmi_design(const double *p1, const double *p2, const double *l1, const do
 
 /* Kernels launched by this library on the calling process so far (bench.py reports it as gpu_launches). */
 int64_t pd_launch_count(void);
-/* Name of the kernel variant pd_decode* uses for this decoder ("generic", "scl_lut_warp", ...). */
+/* Name of the kernel variant pd_decode* uses for this decoder ("scl_lut_warp", "path_warp", "generic", or "path_cta" for
+   every list decoder with L > 32). */
 const char *pd_kernel_name(const pd_decoder *dec);
 /* Why a LUT-class decoder is NOT on "scl_lut_warp" ("" when it is, or for the float / uniform / Lloyd classes): the shape
    rule that sent it to the slower path_warp / generic kernels.  The same text is printed once on stderr at pd_create

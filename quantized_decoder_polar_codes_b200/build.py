@@ -42,6 +42,7 @@ _UNITS = [("capi", "pb_capi.cu", [], None)]          # None = every header
 _UNITS += [("k%d" % t, "pb_kernels.cu", ["-DPB_TU=%d" % t], _COMMON + ["pb_scl_lut.cuh"]) for t in (1, 2, 3, 4)]
 _UNITS += [("k%d" % t, "pb_kernels.cu", ["-DPB_TU=%d" % t], _COMMON + ["pb_path_warp.cuh"]) for t in (5, 6, 7, 8)]
 _UNITS += [("k9", "pb_kernels.cu", ["-DPB_TU=9"], _COMMON)]
+_UNITS += [("k10", "pb_kernels.cu", ["-DPB_TU=10"], _COMMON + ["pb_path_cta.cuh"])]
 _UNITS += [("lutgen", "pb_lutgen.cu", [], ["pb_lutgen.cuh"])]
 OBJDIR = os.path.join(HERE, "build")
 

@@ -28,6 +28,7 @@
 #include "pb_generic.cuh"
 #include "pb_scl_lut.cuh"
 #include "pb_path_warp.cuh"
+#include "pb_path_cta.cuh"
 #ifndef PB_HOST_EMU   // (tools/emu emulates the decode kernels only)
 #include "pb_sim.cuh"
 #include "pb_enc.cuh"
@@ -297,9 +298,11 @@ struct pd_decoder {
     // specialised kernel
     FastPlan fast{};
     PathPlan path{};          // warp-level schedule interpreter (all classes, L power of two)
+    CtaPlan cta{};            // CTA-level schedule interpreter: the list sizes 64, 128, 256, and nothing else runs them
     cudaEvent_t fork_ev = nullptr, join_ev[2] = {nullptr, nullptr};   // pd_decode_device: split of large batches
     cudaStream_t side[2] = {nullptr, nullptr};
-    int force = 0;            // POLAR_B200_FORCE_GENERIC: 1 = CTA-per-frame generic kernel, 2 = path_warp
+    int force = 0;            // POLAR_B200_FORCE_GENERIC: 1 = CTA-per-frame generic kernel, 2 = path_warp (L <= 32 only:
+                              // L > 32 always runs path_cta)
     const char *kernel_name = "generic";
     int *d_err = nullptr;             // device view of the mapped error flag
     volatile int *h_err = nullptr;   // host view
@@ -523,6 +526,12 @@ bool want_path(const pd_decoder *D, int dtype, const void *d_in) {
 
 int launch(pd_decoder *D, const void *d_in, int dtype, int64_t B, uint8_t *d_out, cudaStream_t s, char *ws) {
     if (B <= 0) return PD_OK;
+    if (D->cta.ok) {
+        int rc = launch_path_cta(D->dev, D->cta, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
+        g_launches++;
+        if (rc != 0) return fail(PD_ECUDA, "path_cta launch failed: %s", cudaGetErrorString((cudaError_t)rc));
+        return PD_OK;
+    }
     if (want_fast(D, dtype, d_in)) {
         int rc = launch_fast_lut(D->dev, D->fast, d_in, dtype, B, d_out, s, reinterpret_cast<uint32_t *>(ws), D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
         g_launches++;
@@ -540,6 +549,7 @@ int launch(pd_decoder *D, const void *d_in, int dtype, int64_t B, uint8_t *d_out
 
 // bytes of global workspace the kernel chosen for this call needs
 size_t ws_need(const pd_decoder *D, int dtype, const void *d_in, int64_t B) {
+    if (D->cta.ok) return D->cta.ws_bytes_per_cta * (size_t)path_cta_grid(D->cta, B, D->sm_count);
     if (want_fast(D, dtype, d_in)) return pb::kWsHeadWords * 4 + D->fast.ws_bytes_per_cta * (size_t)fast_grid(D->fast, B, D->sm_count);
     if (want_path(D, dtype, d_in)) return D->path.ws_bytes_per_cta * (size_t)path_grid(D->path, B, D->sm_count);
     return D->use_smem ? 0 : D->ws_bytes * (size_t)generic_grid(D, B);
@@ -547,6 +557,7 @@ size_t ws_need(const pd_decoder *D, int dtype, const void *d_in, int64_t B) {
 
 // frames one full wave of the chosen (persistent) kernel holds in flight; 0 for the CTA-per-frame generic kernel
 int64_t wave_frames(const pd_decoder *D, int dtype, const void *d_in) {
+    if (D->cta.ok) return (int64_t)D->sm_count * D->cta.ctas_per_sm;   // one frame per CTA
     if (want_fast(D, dtype, d_in)) return (int64_t)D->sm_count * D->fast.ctas_per_sm * D->fast.p.warps * (32 >> D->fast.logL);
     if (want_path(D, dtype, d_in)) return (int64_t)D->sm_count * D->path.ctas_per_sm * (32 >> D->path.logL);
     return 0;
@@ -604,7 +615,12 @@ int pd_create(const pd_config *c, pd_decoder **out) {
     int n = 0;
     while ((1 << n) < N) n++;
     const bool list = is_list(kind), fastk = is_fast(kind), ca = is_ca(kind);
-    if (list && (c->L < 1 || c->L > kMaxL)) return fail(PD_EINVAL, "L=%d must be in [1,%d]", c->L, kMaxL);
+    if (list) {   // 1..32 on the warp kernels; 64, 128 and 256 on path_cta, which keeps partial sums as 32-bit words per path
+        const bool big = c->L == 64 || c->L == 128 || c->L == 256;
+        if (c->L < 1 || (c->L > kMaxL && !big) || (big && (N < 32 || kind == PD_BD_CASCL)))
+            return fail(PD_EINVAL, "L=%d: list sizes are 1..%d, or 64, 128 or 256 with N >= 32 (here N=%d; blind-detection CA-SCL: 1..%d only)",
+                        c->L, kMaxL, N, kMaxL);
+    }
     std::vector<int32_t> info_pos;
     for (int i = 0; i < N; ++i) if (c->frozen_bits[i] == 0) info_pos.push_back(i);
     if ((int)info_pos.size() != c->K) return fail(PD_EINVAL, "K=%d but frozen_bits has %zu non-frozen positions", c->K, info_pos.size());
@@ -715,10 +731,15 @@ int pd_create(const pd_config *c, pd_decoder **out) {
         *D->h_err = 0;
         D->d_err = (int *)dp;
     }
-    if ((rc = plan_generic(D))) return bail(rc);
-    plan_path_warp(D->dev, &D->path);
-    if (const char *e = getenv("POLAR_B200_FORCE_GENERIC")) D->force = atoi(e);
-    D->kernel_name = (D->fast.ok && D->force == 0) ? D->fast.name : (D->path.ok && D->force != 1) ? "path_warp" : "generic";
+    if (d.L > kMaxL) {   // path_cta only: the generic kernel's control block and path_warp's lanes stop at 32 paths
+        if (const char *why = plan_path_cta(D->dev, &D->cta)) return bail(fail(PD_ECUDA, "path_cta (N=%d, L=%d): %s", N, d.L, why));
+        D->kernel_name = "path_cta";
+    } else {
+        if ((rc = plan_generic(D))) return bail(rc);
+        plan_path_warp(D->dev, &D->path);
+        if (const char *e = getenv("POLAR_B200_FORCE_GENERIC")) D->force = atoi(e);
+        D->kernel_name = (D->fast.ok && D->force == 0) ? D->fast.name : (D->path.ok && D->force != 1) ? "path_warp" : "generic";
+    }
     // a LUT class that falls off the nibble kernel runs 3-100x slower: say so once per reason (POLAR_B200_QUIET=1 silences it)
     if (d.domain == DOM_LUT && !D->fast.ok && D->force == 0 && *D->fast.why && !getenv("POLAR_B200_QUIET")) {
         static std::mutex mu;

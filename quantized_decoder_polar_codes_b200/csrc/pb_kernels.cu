@@ -4,6 +4,7 @@
 //         2  scl_lut_warp L=8 Fast-SSC variants      6  path_warp float
 //         3  scl_lut_warp L=1,2                      7  path_warp uniform
 //         4  scl_lut_warp L=4                        8  path_warp Lloyd
+//                                                   10  path_cta (L = 64, 128, 256), all domains
 #if PB_TU >= 1 && PB_TU <= 4
 #define PB_TU_SCL
 #include "pb_scl_lut.cuh"
@@ -50,6 +51,12 @@ const void *generic_kernel_fn(int dom, bool l, bool w) {
     }
 }
 }  // namespace pb
+#elif PB_TU == 10
+#define PB_TU_PATH_CTA
+#include "pb_path_cta.cuh"
+namespace pb {
+const void *path_cta_kernel_fn(int dom, int logL) { return path_cta_kernel_fn_all(dom, logL); }
+}  // namespace pb
 #else
-#error "PB_TU must be 1..9"
+#error "PB_TU must be 1..10"
 #endif

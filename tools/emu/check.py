@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Bit-exactness of the decode kernels under the host emulator (tools/emu/build) against the CPU oracle.
-Development tooling: lets kernel changes be checked on the GPU-less build box.  Usage: check.py [case-filter]"""
+Development tooling: lets kernel changes be checked on the GPU-less build box.  Usage: check.py [case-filter]
+(a filter starting with "path_cta" selects the path_cta cases, which the default run leaves out)"""
 import importlib.util
 import os
 import sys
@@ -60,12 +61,34 @@ CASES = [
     ("scl_32", "SCLLUTDecoder", dict(N=32, K=16, L=8, B=40)),
 ]
 
+# path_cta (L = 64, 128, 256): one fiber per path makes these slow under the emulator, so they run only when asked for
+# (`check.py path_cta`, or a filter starting with it), never in the default run.
+CTA_CASES = [
+    ("path_cta_sclut_32", "SCLLUTDecoder", dict(N=32, K=16, L=64, B=48)),
+    ("path_cta_sclut_32_dead", "SCLLUTDecoder", dict(N=32, K=5, L=64, B=48)),      # L > 2^K: dead-path ties to the end
+    ("path_cta_sclut_64", "SCLLUTDecoder", dict(N=64, K=32, L=256, B=24)),
+    ("path_cta_sclut_128m", "SCLLUTDecoder", dict(N=128, K=64, L=64, B=4, tables="minsum", ebn0_db=1.0)),
+    ("path_cta_ca_128", "CASCLLUTDecoder", dict(N=128, K=88, A=64, L=64, B=32)),
+    ("path_cta_ca_64", "CASCLLUTDecoder", dict(N=64, K=40, A=16, L=256, B=16)),
+    ("path_cta_fast_64", "FastSCLLUTDecoder", dict(N=64, K=30, L=64, B=32)),
+    ("path_cta_fast_128", "FastSCLLUTDecoder", dict(N=128, K=64, L=256, B=16)),
+    ("path_cta_float_32", "SCLDecoder", dict(N=32, K=16, L=256, B=3, tables="channel")),
+    ("path_cta_float_128", "SCLDecoder", dict(N=128, K=64, L=64, B=4, tables="channel")),
+    ("path_cta_float_rand", "SCLDecoder", dict(N=64, K=32, L=64, B=32)),
+    ("path_cta_uniform_64", "SCLUniformQuantizedDecoder", dict(N=64, K=32, L=64, B=32)),
+    ("path_cta_lloyd_64", "SCLLloydQuantizedDecoder", dict(N=64, K=32, L=128, B=16)),
+    ("path_cta_fastf_64", "FastSCLDecoder", dict(N=64, K=30, L=128, B=16)),
+    ("path_cta_cafast_64", "CAFastSCLLUTDecoder", dict(N=64, K=54, A=30, L=64, B=16)),
+    ("path_cta_cascl_64", "CASCLDecoder", dict(N=64, K=40, A=16, L=128, B=16, tables="channel")),
+    ("path_cta_uniform_128", "SCLUniformQuantizedDecoder", dict(N=128, K=64, L=256, B=16)),
+]
+
 
 def main():
     flt = sys.argv[1] if len(sys.argv) > 1 else ""
     emu = load_emu()
     bad_total = 0
-    for name, kind, ckw in CASES:
+    for name, kind, ckw in (CTA_CASES if flt.startswith("path_cta") else CASES):
         if flt and flt not in name:
             continue
         ckw = dict(ckw)

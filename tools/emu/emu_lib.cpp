@@ -1,4 +1,4 @@
-// libpolar_b200 built for the host emulator (see shim/cuda_runtime.h): the C ABI + the three decode kernels as plain
+// libpolar_b200 built for the host emulator (see shim/cuda_runtime.h): the C ABI + the four decode kernel families as plain
 // C++, threads as fibers.  Development tooling only; built into tools/emu/build/, never into the package.
 #include <cuda_runtime.h>   // resolves to shim/cuda_runtime.h (-I order)
 
@@ -104,6 +104,7 @@ void launch(const std::function<void()> &body, dim3 grid, dim3 block, size_t sme
 
 #define PB_TU_SCL
 #define PB_TU_PATH
+#define PB_TU_PATH_CTA
 #include "pb_capi.cu"
 
 namespace pb {
@@ -118,6 +119,7 @@ const void *path_fn_lut(int logL) { return path_kernel_fn_d<DOM_LUT>(logL); }
 const void *path_fn_float(int logL) { return path_kernel_fn_d<DOM_FLOAT>(logL); }
 const void *path_fn_uniform(int logL) { return path_kernel_fn_d<DOM_UNIFORM>(logL); }
 const void *path_fn_lloyd(int logL) { return path_kernel_fn_d<DOM_LLOYD>(logL); }
+const void *path_cta_kernel_fn(int dom, int logL) { return path_cta_kernel_fn_all(dom, logL); }
 template <int DOM, bool LIST>
 static const void *generic_fn(bool warp) {
     return warp ? PB_KFN(generic_decode_kernel<DOM, LIST, true>) : PB_KFN(generic_decode_kernel<DOM, LIST, false>);

@@ -111,6 +111,7 @@ struct State {
     std::vector<WarpState> warps;
     std::vector<unsigned> ncoll;   // per thread: collectives executed so far (selects the exchange buffer)
     int blk_arrived = 0, blk_gen = 0;
+    int blk_or[2] = {0, 0};        // __syncthreads_or: one accumulator per barrier generation parity
     char *smem = nullptr;
     std::function<void()> body;
     int live = 0;
@@ -132,6 +133,16 @@ inline void block_barrier() {
     const int g = s.blk_gen;
     if (++s.blk_arrived == s.nthreads) { s.blk_arrived = 0; s.blk_gen++; }
     else while (s.blk_gen == g) yield();
+}
+// generation g accumulates into blk_or[g & 1]; it is cleared by the first arrival at generation g + 2, which no thread
+// reaches before every thread has passed generation g + 1, i.e. has read the result of g
+inline int block_barrier_or(int pred) {
+    State &s = st();
+    const int g = s.blk_gen;
+    if (s.blk_arrived == 0) s.blk_or[g & 1] = 0;
+    s.blk_or[g & 1] |= pred ? 1 : 0;
+    block_barrier();
+    return s.blk_or[g & 1];
 }
 template <class T> inline T exchange(T v, int src) {   // one barrier per collective: double-buffered slots
     static_assert(sizeof(T) <= 8, "shuffle of > 8 bytes");
@@ -175,6 +186,7 @@ static inline cudaError_t cudaLaunchKernel(const void *fn, dim3 grid, dim3 block
 // ------------------------------------------------------------------------------------------------ device intrinsics
 static inline void __syncwarp(unsigned = 0xffffffffu) { pb_emu::warp_barrier(); }
 static inline void __syncthreads() { pb_emu::block_barrier(); }
+static inline int __syncthreads_or(int pred) { return pb_emu::block_barrier_or(pred); }
 template <class T> static inline T __shfl_sync(unsigned, T v, int src, int width = 32) {
     const int l = pb_emu::lane();
     return pb_emu::exchange(v, (l & ~(width - 1)) | (src & (width - 1)));
