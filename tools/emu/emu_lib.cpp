@@ -145,6 +145,22 @@ extern "C" int pb_emu_fast_plan(const pd_decoder *dec, int *hist, int *n_ops, in
     return 0;
 }
 
+// The plan of a decoder on scl_lut_warp in full: its op entries (x, y pairs) into ops[2 * ops_cap], the value-level
+// layout (voff[kMaxLog + 2] and gl), and the uploaded stream, head copies included, into stream[stream_cap] with its
+// length in words in *stream_words.  Returns the number of ops, or -1 when the decoder is not on scl_lut_warp.
+extern "C" int pb_emu_fast_plan_detail(const pd_decoder *dec, uint32_t *ops, int ops_cap, int *voff, int *gl,
+                                       uint32_t *stream, long long stream_cap, long long *stream_words) {
+    if (!dec->fast.ok) return -1;
+    const std::vector<uint2> &o = dec->fast.ops;
+    for (int i = 0; i < (int)o.size() && i < ops_cap; ++i) { ops[2 * i] = o[i].x; ops[2 * i + 1] = o[i].y; }
+    for (int d = 0; d < pb::kMaxLog + 2; ++d) voff[d] = dec->fast.p.voff[d];
+    *gl = dec->fast.p.gl;
+    const long long words = ((long long)dec->fast.p.n_chunks + pb::kRingChunks - 1) * 128;
+    *stream_words = words;
+    memcpy(stream, dec->fast.p.stream, (size_t)std::min(words, stream_cap) * 4);
+    return (int)o.size();
+}
+
 // entry points of the real library that the emulator does not provide (the pybind module links them)
 extern "C" {
 int pd_count_errors(const uint8_t *, const uint8_t *, int64_t, int32_t, unsigned long long *, void *) { return PD_ECUDA; }
