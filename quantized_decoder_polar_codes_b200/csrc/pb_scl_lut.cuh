@@ -69,7 +69,8 @@ struct FastParams {
     const uint32_t *crc_rem;       // [A] CRC remainder of each unit message bit (CA kinds)
     uint32_t crc_checkmask;
     int warps;                     // decoding warps per CTA
-    int dbg;                       // POLAR_B200_KDEBUG: 1 = never take the sorted-keeps shortcut in fork (A/B measurements)
+    int dbg;                       // POLAR_B200_KDEBUG bits (A/B measurements): 1 = never take the sorted-keeps shortcut
+                                   // in fork (and so its identity exit), 2 = never take the identity exit in fork
     int reserved[2];               // unused: keeps the offsets of the fields below, which the kernels' register allocation
                                    // (and so the occupancy and pd_wave_frames) follows -- without it the L=1 kernel of
                                    // SCLUTDecoder drops from 61 to 56 registers and gets a different wave size
@@ -122,6 +123,11 @@ inline std::map<size_t, Slot> &slots() { static std::map<size_t, Slot> m; return
 inline unsigned long long *counts() { static unsigned long long c[2 * 1024] = {}; return c + 2 * pb_emu::st().cur; }   // issued, waited
 inline void forget(smaddr_t lane_slot0) { for (int k = 0; k < kRingChunks; ++k) slots().erase(lane_slot0 + k * 512u); }
 }  // namespace emu_ring
+// forks seen and identity exits taken (see fork), counted once per warp
+namespace emu_fork {
+inline unsigned long long &seen() { static unsigned long long n = 0; return n; }
+inline unsigned long long &taken() { static unsigned long long n = 0; return n; }
+}  // namespace emu_fork
 __device__ __forceinline__ void cp_async16(smaddr_t dst, const void *gsrc) {
     emu_ring::Slot &s = emu_ring::slots()[dst];
     if (s.unread) { fprintf(stderr, "scl_lut_warp: ring slot refilled before its chunk was read\n"); abort(); }
@@ -497,7 +503,26 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
         // the metrics in rank order (slot r = r-th smallest key, equal keys in index order), so (keep_j, j) < (K0, me) is
         // exactly j < me: that part of the rank is `me`, and a third of the compares goes away.  Uniform over the warp
         // (it follows the frozen pattern, not the data).
+        // Identity exit: with the keeps sorted, every flip key that is >= the largest keep K0[L-1] ranks after all keeps
+        // (on a tie its index L+j is larger), so when that holds on every lane the survivors are the keeps in their slots:
+        // p = lane, fl = 0, and PM, the pointer words and the subtree registers stay.  Exact, the same fp64 compares
+        // as the rank; most forks of a frame's later leaves take it.
         auto fork = [&](double K0, double K1, int &p, uint32_t &fl, bool keeps_sorted) {
+#ifdef PB_HOST_EMU
+            if (lane == 0) emu_fork::seen()++;
+#endif
+            if (!FAST && L > 1 && keeps_sorted && !(fp.dbg & 2)) {
+                const double Klast = __shfl_sync(kFull, K0, gbase | (L - 1));
+                if (__all_sync(kFull, K1 >= Klast)) {
+#ifdef PB_HOST_EMU
+                    if (lane == 0) emu_fork::taken()++;
+                    if (!(__shfl_sync(kFull, K0, me > 0 ? lane - 1 : lane) <= K0)) { fprintf(stderr, "scl_lut_warp: identity exit on unsorted metrics\n"); abort(); }
+#endif
+                    p = lane;
+                    fl = 0;
+                    return;
+                }
+            }
             __syncwarp();
             *reinterpret_cast<double2 *>(&KS[(me * FPW + grp) * 2]) = make_double2(K0, K1);
             __syncwarp();

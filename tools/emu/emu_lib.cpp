@@ -161,6 +161,13 @@ extern "C" int pb_emu_fast_plan_detail(const pd_decoder *dec, uint32_t *ops, int
     return (int)o.size();
 }
 
+// The fork counters of scl_lut_warp, once per warp: forks seen and identity exits taken since the last reset.
+extern "C" void pb_emu_fork_counts(unsigned long long *seen, unsigned long long *taken, int reset) {
+    *seen = pb::emu_fork::seen();
+    *taken = pb::emu_fork::taken();
+    if (reset) pb::emu_fork::seen() = pb::emu_fork::taken() = 0;
+}
+
 // entry points of the real library that the emulator does not provide (the pybind module links them)
 extern "C" {
 int pd_count_errors(const uint8_t *, const uint8_t *, int64_t, int32_t, unsigned long long *, void *) { return PD_ECUDA; }
