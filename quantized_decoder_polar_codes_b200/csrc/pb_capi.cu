@@ -15,6 +15,7 @@
 #include <condition_variable>
 #include <functional>
 #include <limits>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -128,6 +129,59 @@ struct StreamSlot {
     size_t h_in_cap = 0, h_out_cap = 0;
     cudaEvent_t done = nullptr;
 };
+
+// Grow-only buffers: reallocated, contents dropped, when a call needs more than the capacity.  The caller makes sure no
+// work in flight still uses the old buffer.
+template <typename T>
+cudaError_t grow(T **p, size_t *cap, size_t need) {
+    if (need <= *cap) return cudaSuccess;
+    cudaFree(*p);
+    *p = nullptr; *cap = 0;
+    const cudaError_t e = cudaMalloc((void **)p, need);
+    if (e == cudaSuccess) *cap = need;
+    return e;
+}
+template <typename T>
+cudaError_t grow_pinned(T **p, size_t *cap, size_t need) {
+    if (need <= *cap) return cudaSuccess;
+    if (*p) cudaFreeHost(*p);
+    *p = nullptr; *cap = 0;
+    const cudaError_t e = cudaHostAlloc((void **)p, need, cudaHostAllocPortable);
+    if (e == cudaSuccess) *cap = need;
+    return e;
+}
+
+// scratch device buffers of one call, freed when it returns
+struct DevBufs {
+    std::vector<void *> v;
+    ~DevBufs() { for (void *p : v) cudaFree(p); }
+    template <class T> T *get(size_t n) {
+        void *p = nullptr;
+        if (cudaMalloc(&p, std::max<size_t>(n * sizeof(T), 16)) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+        v.push_back(p);
+        return reinterpret_cast<T *>(p);
+    }
+};
+
+// makes `device` current; PD_ECUDA without any CUDA device, PD_EINVAL for an id outside the box
+int probe_device(int device) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(PD_ECUDA, "no CUDA device: libpolar_b200 has no CPU path");
+    if (device < 0 || device >= ndev) return fail(PD_EINVAL, "device %d out of range", device);
+    CUDA_TRY(cudaSetDevice(device));
+    return PD_OK;
+}
+
+// Generator taps below the leading term of the CRC polynomial with the exponents loc[0..n) (crc_p), bit crc_n-1 for
+// x^1 down to bit 0 for x^crc_n; false when an exponent is outside [0, crc_n].
+bool crc_taps(int crc_n, const int32_t *loc, int n, uint32_t *taps) {
+    *taps = 0;
+    for (int i = 0; i < n; ++i) {
+        if (loc[i] < 0 || loc[i] > crc_n) return false;
+        if (loc[i] > 0) *taps |= 1u << (crc_n - loc[i]);
+    }
+    return true;
+}
 
 }  // namespace
 
@@ -290,12 +344,7 @@ struct pd_decoder {
     std::vector<void *> allocs;
     std::vector<Step> steps;
     int64_t elem_ops = 0, n_sorts = 0;
-    // generic kernel launch geometry
-    int threads = 32;
-    size_t ws_bytes = 0;      // per-CTA workspace
-    int use_smem = 0;
-    int ctas_per_sm = 1;
-    // specialised kernel
+    GenericPlan generic{};    // CTA-per-frame kernel (L <= 32)
     FastPlan fast{};
     PathPlan path{};          // warp-level schedule interpreter (all classes, L power of two)
     CtaPlan cta{};            // CTA-level schedule interpreter: the list sizes 64, 128, 256, and nothing else runs them
@@ -303,7 +352,6 @@ struct pd_decoder {
     cudaStream_t side[2] = {nullptr, nullptr};
     int force = 0;            // POLAR_B200_FORCE_GENERIC: 1 = CTA-per-frame generic kernel, 2 = path_warp (L <= 32 only:
                               // L > 32 always runs path_cta)
-    const char *kernel_name = "generic";
     int *d_err = nullptr;             // device view of the mapped error flag
     volatile int *h_err = nullptr;   // host view
     double *dbg_pm = nullptr;
@@ -324,17 +372,6 @@ struct pd_decoder {
 constexpr size_t kSmallIn = 64 << 10, kSmallOut = 16 << 10;   // bytes of input / output served by the mapped path
 
 namespace {
-
-template <typename T>
-int upload(pd_decoder *D, const std::vector<T> &h, const T **out) {
-    void *p = nullptr;
-    size_t bytes = std::max<size_t>(h.size() * sizeof(T), 16);
-    CUDA_TRY(cudaMalloc(&p, bytes));
-    D->allocs.push_back(p);
-    if (!h.empty()) CUDA_TRY(cudaMemcpy(p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice));
-    *out = reinterpret_cast<const T *>(p);
-    return PD_OK;
-}
 
 bool special_type(int kind, int t) {
     if (!is_fast(kind)) return false;
@@ -452,11 +489,10 @@ int build_lut(pd_decoder *D, const pd_config *c) {
         loff[r] = (uint32_t)c->llr_off[r];
     }
     std::vector<double> llr(c->llr_pool, c->llr_pool + total);
-    int rc;
-    if ((rc = upload(D, pool, &D->dev.lut))) return rc;
-    if ((rc = upload(D, tabs, &D->dev.tabs))) return rc;
-    if ((rc = upload(D, llr, &D->dev.llr))) return rc;
-    if ((rc = upload(D, loff, &D->dev.llr_off))) return rc;
+    CUDA_TRY(upload(D->allocs, pool.data(), pool.size(), &D->dev.lut));
+    CUDA_TRY(upload(D->allocs, tabs.data(), tabs.size(), &D->dev.tabs));
+    CUDA_TRY(upload(D->allocs, llr.data(), llr.size(), &D->dev.llr));
+    CUDA_TRY(upload(D->allocs, loff.data(), loff.size(), &D->dev.llr_off));
     {
         const bool fastk = is_fast(kind);
         const int max_special = !fastk ? -1 : (is_list(kind) ? 2 : 3);
@@ -465,102 +501,57 @@ int build_lut(pd_decoder *D, const pd_config *c) {
     return PD_OK;
 }
 
-// kernel instantiations live in pb_kernels.cu (one object per family, compiled in parallel)
-const void *generic_fn_for(const pd_decoder *D) {
-    return pb::generic_kernel_fn(D->dev.domain, D->dev.list != 0, D->threads == 32);
-}
-
-int generic_grid(const pd_decoder *D, int64_t B) {
-    int64_t g = (int64_t)D->sm_count * D->ctas_per_sm;
-    return (int)std::max<int64_t>(1, std::min<int64_t>(g, B));
-}
-
-int launch_generic(pd_decoder *D, const void *d_in, int dtype, int64_t B, uint8_t *d_out, cudaStream_t s, char *ws) {
-    int grid = generic_grid(D, B);
-    size_t smem = D->use_smem ? D->ws_bytes : 0;
-    long long Bll = B;
-    void *args[] = {(void *)&D->dev, (void *)&d_in, (void *)&dtype, (void *)&d_out, (void *)&Bll, (void *)&ws, (void *)&D->ws_bytes,
-                    (void *)&D->use_smem, (void *)&D->d_err, (void *)&D->dbg_pm, (void *)&D->dbg_win};
-    CUDA_TRY(cudaLaunchKernel(generic_fn_for(D), dim3(grid), dim3(D->threads), args, smem, s));
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    return PD_OK;
-}
-
-int plan_generic(pd_decoder *D) {
-    const Dev &d = D->dev;
-    int L = d.list ? d.L : 1;
-    size_t vsz = d.domain == DOM_LUT ? 1 : 8;
-    size_t ws = (((size_t)L * d.N * vsz + 15) & ~(size_t)15) + (size_t)L * d.r1_tmax * (8 + 4) + (size_t)L * 3 * d.N + (size_t)2 * L * d.r1_tmax + d.N;
-    ws = (ws + 15) & ~(size_t)15;
-    D->ws_bytes = ws;
-    int64_t work = (int64_t)L * d.N / 2;
-    int th = 32;
-    while (th < 256 && th * 8 < work) th *= 2;
-    D->threads = th;
-    D->use_smem = ws <= 96 * 1024;
-    const void *fn = generic_fn_for(D);
-    // (the attribute belongs to the kernel function, which every decoder of the same domain shares: always the cap, never
-    //  this decoder's own size -- a smaller decoder created later must not shrink it under a live larger one)
-    if (D->use_smem) CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-    int occ = 0;
-    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, th, D->use_smem ? ws : 0));
-    if (occ < 1) return fail(PD_ECUDA, "generic kernel does not fit on the device (ws=%zu)", ws);
-    D->ctas_per_sm = occ;
-    return PD_OK;
-}
-
-size_t ws_need(const pd_decoder *D, int dtype, const void *d_in, int64_t B);
-bool want_fast(const pd_decoder *D, int dtype, const void *d_in) {
-    if (D->fast.ok && dtype != PD_F64 && D->force == 0 && (reinterpret_cast<uintptr_t>(d_in) & 15u) != 0) {
+// The kernel family that runs a call with `dtype` symbols at `d_in` (nullptr: a buffer of the library's own, which
+// cudaMalloc aligns).  scl_lut_warp reads its input with 16-byte loads and takes symbols only.
+enum class Route { Cta, Lut, Path, Generic };
+constexpr const char *kRouteName[] = {"path_cta", "scl_lut_warp", "path_warp", "generic"};
+Route route(const pd_decoder *D, int dtype, const void *d_in) {
+    if (D->cta.ok) return Route::Cta;
+    if (D->fast.ok && dtype != PD_F64 && D->force == 0) {
+        if ((reinterpret_cast<uintptr_t>(d_in) & 15u) == 0) return Route::Lut;
         static std::atomic<bool> told{false};
         if (!told.exchange(true) && !getenv("POLAR_B200_QUIET"))
             fprintf(stderr, "[polar_b200] note: input pointer %p is not 16-byte aligned: this call runs on the slower 'path_warp' / 'generic' kernel\n", d_in);
-        return false;
     }
-    return D->fast.ok && dtype != PD_F64 && D->force == 0;
-}
-bool want_path(const pd_decoder *D, int dtype, const void *d_in) {
-    return !want_fast(D, dtype, d_in) && D->path.ok && D->force != 1;
+    if (D->path.ok && D->force != 1) return Route::Path;
+    return Route::Generic;
 }
 
-int launch(pd_decoder *D, const void *d_in, int dtype, int64_t B, uint8_t *d_out, cudaStream_t s, char *ws) {
+int launch(pd_decoder *D, Route r, const void *d_in, int dtype, int64_t B, uint8_t *d_out, cudaStream_t s, char *ws) {
     if (B <= 0) return PD_OK;
-    if (D->cta.ok) {
-        int rc = launch_path_cta(D->dev, D->cta, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
-        g_launches++;
-        if (rc != 0) return fail(PD_ECUDA, "path_cta launch failed: %s", cudaGetErrorString((cudaError_t)rc));
-        return PD_OK;
+    const Dev &d = D->dev;
+    int rc;
+    switch (r) {
+    case Route::Cta: rc = launch_path_cta(d, D->cta, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count); break;
+    case Route::Lut:
+        rc = launch_fast_lut(d, D->fast, d_in, dtype, B, d_out, s, reinterpret_cast<uint32_t *>(ws), D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
+        break;
+    case Route::Path: rc = launch_path_warp(d, D->path, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count); break;
+    default: rc = launch_generic(d, D->generic, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count); break;
     }
-    if (want_fast(D, dtype, d_in)) {
-        int rc = launch_fast_lut(D->dev, D->fast, d_in, dtype, B, d_out, s, reinterpret_cast<uint32_t *>(ws), D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
-        g_launches++;
-        if (rc != 0) return fail(PD_ECUDA, "fast kernel launch failed: %s", cudaGetErrorString((cudaError_t)rc));
-        return PD_OK;
-    }
-    if (want_path(D, dtype, d_in)) {
-        int rc = launch_path_warp(D->dev, D->path, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
-        g_launches++;
-        if (rc != 0) return fail(PD_ECUDA, "path_warp launch failed: %s", cudaGetErrorString((cudaError_t)rc));
-        return PD_OK;
-    }
-    return launch_generic(D, d_in, dtype, B, d_out, s, ws);
+    g_launches++;
+    if (rc != 0) return fail(PD_ECUDA, "%s launch failed: %s", kRouteName[(int)r], cudaGetErrorString((cudaError_t)rc));
+    return PD_OK;
 }
 
-// bytes of global workspace the kernel chosen for this call needs
-size_t ws_need(const pd_decoder *D, int dtype, const void *d_in, int64_t B) {
-    if (D->cta.ok) return D->cta.ws_bytes_per_cta * (size_t)path_cta_grid(D->cta, B, D->sm_count);
-    if (want_fast(D, dtype, d_in)) return pb::kWsHeadWords * 4 + D->fast.ws_bytes_per_cta * (size_t)fast_grid(D->fast, B, D->sm_count);
-    if (want_path(D, dtype, d_in)) return D->path.ws_bytes_per_cta * (size_t)path_grid(D->path, B, D->sm_count);
-    return D->use_smem ? 0 : D->ws_bytes * (size_t)generic_grid(D, B);
+// bytes of global workspace a launch over B frames needs
+size_t ws_need(const pd_decoder *D, Route r, int64_t B) {
+    switch (r) {
+    case Route::Cta: return D->cta.ws_bytes_per_cta * (size_t)path_cta_grid(D->cta, B, D->sm_count);
+    case Route::Lut: return pb::kWsHeadWords * 4 + D->fast.ws_bytes_per_cta * (size_t)fast_grid(D->fast, B, D->sm_count);
+    case Route::Path: return D->path.ws_bytes_per_cta * (size_t)path_grid(D->path, B, D->sm_count);
+    default: return D->generic.use_smem ? 0 : D->generic.ws_bytes * (size_t)generic_grid(D->generic, B, D->sm_count);
+    }
 }
 
-// frames one full wave of the chosen (persistent) kernel holds in flight; 0 for the CTA-per-frame generic kernel
-int64_t wave_frames(const pd_decoder *D, int dtype, const void *d_in) {
-    if (D->cta.ok) return (int64_t)D->sm_count * D->cta.ctas_per_sm;   // one frame per CTA
-    if (want_fast(D, dtype, d_in)) return (int64_t)D->sm_count * D->fast.ctas_per_sm * D->fast.p.warps * (32 >> D->fast.logL);
-    if (want_path(D, dtype, d_in)) return (int64_t)D->sm_count * D->path.ctas_per_sm * (32 >> D->path.logL);
-    return 0;
+// frames one full wave of the (persistent) kernel holds in flight; 0 for the CTA-per-frame generic kernel
+int64_t wave_frames(const pd_decoder *D, Route r) {
+    switch (r) {
+    case Route::Cta: return (int64_t)D->sm_count * D->cta.ctas_per_sm;   // one frame per CTA
+    case Route::Lut: return (int64_t)D->sm_count * D->fast.ctas_per_sm * D->fast.p.warps * (32 >> D->fast.logL);
+    case Route::Path: return (int64_t)D->sm_count * D->path.ctas_per_sm * (32 >> D->path.logL);
+    default: return 0;
+    }
 }
 
 size_t dtype_size(int t) { return t == PD_U8 ? 1 : t == PD_I32 ? 4 : 8; }
@@ -571,6 +562,18 @@ int check_dtype(const pd_decoder *D, int t, bool host_call = false) {
         if (t != PD_U8 && t != PD_I32) return fail(PD_EINVAL, "LUT decoders take PD_U8 or PD_I32 symbols (pd_decode also PD_F64-typed symbols)");
     } else if (t != PD_F64) {
         return fail(PD_EINVAL, "float/uniform/Lloyd decoders take PD_F64 LLRs");
+    }
+    return PD_OK;
+}
+
+// the arguments both blind-detection entry points take (host or device pointers alike)
+int check_bd(const pd_decoder *D, const double *llr, int64_t B, const int32_t *rnti, int32_t rnti_len, const uint8_t *bits,
+             const double *metric, const uint8_t *pass) {
+    if (!D || (B > 0 && (!llr || !metric))) return fail(PD_EINVAL, "null argument");
+    if (D->dev.bd == 0) return fail(PD_EINVAL, "pd_decode_bd: the decoder is not a PD_BD_* kind");
+    if (D->dev.bd == 2) {
+        if (B > 0 && (!bits || !pass)) return fail(PD_EINVAL, "null argument");
+        if (rnti_len < 0 || rnti_len > D->dev.crc_n || (rnti_len > 0 && !rnti)) return fail(PD_EINVAL, "RNTI length %d must be in [0,crc_n=%d]", rnti_len, D->dev.crc_n);
     }
     return PD_OK;
 }
@@ -633,37 +636,29 @@ int pd_create(const pd_config *c, pd_decoder **out) {
     uint32_t taps = 0;
     if (ca) {
         if (c->A < 1 || c->A > c->K) return fail(PD_EINVAL, "A=%d must be in [1,K]", c->A);
-        std::vector<int> poly;
         if (kind == PD_CASCL || kind == PD_BD_CASCL) {   // honours the ctor polynomial, compares crc_n bits (PD/src/CASCLDecoder.cpp:49-53,222; CASCLWithRNTI.cpp:48-56,228-233)
             crc_n = c->crc_n;
             if (crc_n < 1 || crc_n > 32) return fail(PD_EINVAL, "crc_n=%d unsupported (1..32)", crc_n);
-            poly.assign(crc_n + 1, 0);
-            for (int i = 0; i < c->crc_loc_len; ++i) {
-                if (c->crc_loc[i] < 0 || c->crc_loc[i] > crc_n) return fail(PD_EINVAL, "crc_p entry out of range");
-                poly[c->crc_loc[i]] = 1;
-            }
+            if (!crc_taps(crc_n, c->crc_loc, c->crc_loc_len, &taps)) return fail(PD_EINVAL, "crc_p entry out of range");
             crc_check = crc_n;
         } else {                  // hard-coded CRC-24, compares K-A bits (PD/include/CASCLLUTDecoder.h:33-34, CASCLLUTDecoder.cpp:280)
-            static const int loc[13] = {24, 23, 21, 20, 17, 15, 13, 12, 8, 4, 2, 1, 0};
+            static const int32_t loc[13] = {24, 23, 21, 20, 17, 15, 13, 12, 8, 4, 2, 1, 0};
             crc_n = 24;
-            poly.assign(25, 0);
-            for (int l : loc) poly[l] = 1;
+            crc_taps(crc_n, loc, 13, &taps);
             crc_check = c->K - c->A;
             if (crc_check > 24) return fail(PD_EINVAL, "K-A=%d > 24: the reference reads past its 24 check bits", crc_check);
         }
         if (c->A + crc_check > c->K) return fail(PD_EINVAL, "A + checked CRC bits exceeds K");
-        for (int k = 0; k < crc_n; ++k) if (poly[1 + k]) taps |= 1u << (crc_n - 1 - k);
     }
 
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(PD_ECUDA, "no CUDA device: libpolar_b200 has no CPU path");
-    if (c->device < 0 || c->device >= ndev) return fail(PD_EINVAL, "device %d out of range", c->device);
-    CUDA_TRY(cudaSetDevice(c->device));
+    int rc = probe_device(c->device);
+    if (rc) return rc;
     cudaDeviceProp prop;
     CUDA_TRY(cudaGetDeviceProperties(&prop, c->device));
     if (prop.major != 10) return fail(PD_ECUDA, "device %d is sm_%d%d; this library is built for sm_100a only", c->device, prop.major, prop.minor);
 
     pd_decoder *D = new pd_decoder();
+    std::unique_ptr<pd_decoder, void (*)(pd_decoder *)> own(D, pd_destroy);   // frees D on every error return
     D->device = c->device;
     D->sm_count = prop.multiProcessorCount;
     Dev &d = D->dev;
@@ -681,81 +676,81 @@ int pd_create(const pd_config *c, pd_decoder **out) {
     D->elem_ops = b.elem_ops; D->n_sorts = b.n_sorts;
     d.r1_tmax = b.r1_tmax;
     d.n_steps = (int)b.steps.size();
-    int rc = PD_OK;
-    auto bail = [&](int code) { pd_destroy(D); return code; };
-    if ((rc = upload(D, b.steps, &d.steps))) return bail(rc);
-    if ((rc = upload(D, info_pos, &d.info_pos))) return bail(rc);
+    CUDA_TRY(upload(D->allocs, b.steps.data(), b.steps.size(), &d.steps));
+    CUDA_TRY(upload(D->allocs, info_pos.data(), info_pos.size(), &d.info_pos));
 
     if (d.domain == DOM_LUT) {
-        if ((rc = build_lut(D, c))) return bail(rc);
+        if ((rc = build_lut(D, c))) return rc;
     } else if (d.domain == DOM_UNIFORM) {
-        if (!c->decoder_r_f || !c->decoder_r_g) return bail(fail(PD_EINVAL, "decoder_r_f / decoder_r_g missing"));
-        std::vector<double> rf(c->decoder_r_f, c->decoder_r_f + N - 1), rg(c->decoder_r_g, c->decoder_r_g + N - 1);
-        for (int i = 0; i < N - 1; ++i)
-            if (!(rf[i] > 0) || !(rg[i] > 0) || !std::isfinite(rf[i]) || !std::isfinite(rg[i]))
-                return bail(fail(PD_EINVAL, "decoder_r_f / decoder_r_g[%d] must be finite and > 0", i));
-        if (c->v < 2) return bail(fail(PD_EINVAL, "v=%d must be >= 2", c->v));
-        if ((rc = upload(D, rf, &d.r_f)) || (rc = upload(D, rg, &d.r_g))) return bail(rc);
+        if (!c->decoder_r_f || !c->decoder_r_g) return fail(PD_EINVAL, "decoder_r_f / decoder_r_g missing");
+        for (int i = 0; i < N - 1; ++i) {
+            const double rf = c->decoder_r_f[i], rg = c->decoder_r_g[i];
+            if (!(rf > 0) || !(rg > 0) || !std::isfinite(rf) || !std::isfinite(rg))
+                return fail(PD_EINVAL, "decoder_r_f / decoder_r_g[%d] must be finite and > 0", i);
+        }
+        if (c->v < 2) return fail(PD_EINVAL, "v=%d must be >= 2", c->v);
+        CUDA_TRY(upload(D->allocs, c->decoder_r_f, N - 1, &d.r_f));
+        CUDA_TRY(upload(D->allocs, c->decoder_r_g, N - 1, &d.r_g));
         d.mf_mul = double(c->v / 2 - 0.5);
         d.mg_mul = double(c->v / 2 - 1);
     } else if (d.domain == DOM_LLOYD) {
-        if (!c->boundaries_f || !c->boundaries_g || !c->reconstruction_f || !c->reconstruction_g) return bail(fail(PD_EINVAL, "Lloyd tables missing"));
-        if (c->n_boundaries < 1 || c->n_reconstruction < 1) return bail(fail(PD_EINVAL, "Lloyd table widths missing"));
+        if (!c->boundaries_f || !c->boundaries_g || !c->reconstruction_f || !c->reconstruction_g) return fail(PD_EINVAL, "Lloyd tables missing");
+        if (c->n_boundaries < 1 || c->n_reconstruction < 1) return fail(PD_EINVAL, "Lloyd table widths missing");
         // bisect() returns reconstruction[lo-1] with lo in [0, n_boundaries] (PD/src/utils.cpp:12-24): the reference reads
         // out of bounds unless the first boundary is below every input and there is a cell per boundary gap
-        if (c->n_reconstruction < c->n_boundaries - 1) return bail(fail(PD_EINVAL, "Lloyd tables: %d reconstruction values for %d boundaries (need >= boundaries-1)", c->n_reconstruction, c->n_boundaries));
+        if (c->n_reconstruction < c->n_boundaries - 1) return fail(PD_EINVAL, "Lloyd tables: %d reconstruction values for %d boundaries (need >= boundaries-1)", c->n_reconstruction, c->n_boundaries);
         for (int t = 0; t < 2; ++t) {
             const double *bd = t ? c->boundaries_g : c->boundaries_f;
             for (int p = 0; p < N - 1; ++p) {
                 const double *row = bd + (size_t)p * c->n_boundaries;
                 for (int k = 0; k < c->n_boundaries; ++k) {
-                    if (row[k] != row[k]) return bail(fail(PD_EINVAL, "boundaries_%s[%d][%d] is NaN", t ? "g" : "f", p, k));
-                    if (k && row[k] < row[k - 1]) return bail(fail(PD_EINVAL, "boundaries_%s[%d] must ascend", t ? "g" : "f", p));
+                    if (row[k] != row[k]) return fail(PD_EINVAL, "boundaries_%s[%d][%d] is NaN", t ? "g" : "f", p, k);
+                    if (k && row[k] < row[k - 1]) return fail(PD_EINVAL, "boundaries_%s[%d] must ascend", t ? "g" : "f", p);
                 }
-                if (!(row[0] <= -1e290)) return bail(fail(PD_EINVAL, "boundaries_%s[%d][0] must be the -1e300 sentinel of LloydQuantizer.py:64 (a value below it reads reconstruction[-1] in the reference)", t ? "g" : "f", p));
-                if (c->n_reconstruction < c->n_boundaries && !(row[c->n_boundaries - 1] >= 1e290)) return bail(fail(PD_EINVAL, "boundaries_%s[%d]: last boundary must be the +1e300 sentinel when there are fewer reconstruction values than boundaries", t ? "g" : "f", p));
+                if (!(row[0] <= -1e290)) return fail(PD_EINVAL, "boundaries_%s[%d][0] must be the -1e300 sentinel of LloydQuantizer.py:64 (a value below it reads reconstruction[-1] in the reference)", t ? "g" : "f", p);
+                if (c->n_reconstruction < c->n_boundaries && !(row[c->n_boundaries - 1] >= 1e290)) return fail(PD_EINVAL, "boundaries_%s[%d]: last boundary must be the +1e300 sentinel when there are fewer reconstruction values than boundaries", t ? "g" : "f", p);
             }
         }
-        size_t nbs = (size_t)(N - 1) * c->n_boundaries, nrs = (size_t)(N - 1) * c->n_reconstruction;
-        std::vector<double> bf(c->boundaries_f, c->boundaries_f + nbs), bg(c->boundaries_g, c->boundaries_g + nbs);
-        std::vector<double> rf(c->reconstruction_f, c->reconstruction_f + nrs), rg(c->reconstruction_g, c->reconstruction_g + nrs);
-        if ((rc = upload(D, bf, &d.bnd_f)) || (rc = upload(D, bg, &d.bnd_g)) || (rc = upload(D, rf, &d.rec_f)) || (rc = upload(D, rg, &d.rec_g))) return bail(rc);
+        const size_t nbs = (size_t)(N - 1) * c->n_boundaries, nrs = (size_t)(N - 1) * c->n_reconstruction;
+        CUDA_TRY(upload(D->allocs, c->boundaries_f, nbs, &d.bnd_f));
+        CUDA_TRY(upload(D->allocs, c->boundaries_g, nbs, &d.bnd_g));
+        CUDA_TRY(upload(D->allocs, c->reconstruction_f, nrs, &d.rec_f));
+        CUDA_TRY(upload(D->allocs, c->reconstruction_g, nrs, &d.rec_g));
         d.nb = c->n_boundaries; d.nr = c->n_reconstruction;
     }
     {   // error flag in mapped pinned host memory: the kernels write it (over PCIe) only when a symbol is out of range,
         // the host reads it without a device->host copy
         void *hp = nullptr, *dp = nullptr;
         if (cudaHostAlloc(&hp, sizeof(int), cudaHostAllocMapped) != cudaSuccess || cudaHostGetDevicePointer(&dp, hp, 0) != cudaSuccess)
-            return bail(fail(PD_ECUDA, "cudaHostAlloc (mapped) failed"));
+            return fail(PD_ECUDA, "cudaHostAlloc (mapped) failed");
         D->h_err = (volatile int *)hp;
         *D->h_err = 0;
         D->d_err = (int *)dp;
     }
     if (d.L > kMaxL) {   // path_cta only: the generic kernel's control block and path_warp's lanes stop at 32 paths
-        if (const char *why = plan_path_cta(D->dev, &D->cta)) return bail(fail(PD_ECUDA, "path_cta (N=%d, L=%d): %s", N, d.L, why));
-        D->kernel_name = "path_cta";
+        if (const char *why = plan_path_cta(D->dev, &D->cta)) return fail(PD_ECUDA, "path_cta (N=%d, L=%d): %s", N, d.L, why);
     } else {
-        if ((rc = plan_generic(D))) return bail(rc);
+        CUDA_TRY(plan_generic(D->dev, &D->generic));
+        if (D->generic.ctas_per_sm < 1) return fail(PD_ECUDA, "generic kernel does not fit on the device (ws=%zu)", D->generic.ws_bytes);
         plan_path_warp(D->dev, &D->path);
         if (const char *e = getenv("POLAR_B200_FORCE_GENERIC")) D->force = atoi(e);
-        D->kernel_name = (D->fast.ok && D->force == 0) ? D->fast.name : (D->path.ok && D->force != 1) ? "path_warp" : "generic";
     }
     // a LUT class that falls off the nibble kernel runs 3-100x slower: say so once per reason (POLAR_B200_QUIET=1 silences it)
-    if (d.domain == DOM_LUT && !D->fast.ok && D->force == 0 && *D->fast.why && !getenv("POLAR_B200_QUIET")) {
+    if (D->force == 0 && *pd_kernel_note(D) && !getenv("POLAR_B200_QUIET")) {
         static std::mutex mu;
         static std::vector<std::string> seen;
         std::lock_guard<std::mutex> lk(mu);
-        const std::string key = std::string(D->fast.why) + "/" + D->kernel_name;
+        const std::string key = std::string(D->fast.why) + "/" + pd_kernel_name(D);
         if (std::find(seen.begin(), seen.end(), key) == seen.end()) {
             seen.push_back(key);
             fprintf(stderr, "[polar_b200] note: this LUT decoder (N=%d, L=%d) runs on the '%s' kernel, not 'scl_lut_warp': %s\n",
-                    N, d.list ? d.L : 1, D->kernel_name, D->fast.why);
+                    N, d.list ? d.L : 1, pd_kernel_name(D), D->fast.why);
         }
     }
     size_t in_frame = (size_t)N * (d.domain == DOM_LUT ? 4 : 8);
     D->chunk_frames = std::max<int64_t>(1024, (int64_t)((32u << 20) / in_frame));
     D->cfg.take(c);
-    *out = D;
+    *out = own.release();
     return PD_OK;
 }
 
@@ -810,9 +805,10 @@ int pd_counters_allreduce(pd_decoder *D, unsigned long long *const *dev_counters
 }
 
 int pd_out_len(const pd_decoder *D) { return D ? D->dev.Kout : 0; }
-int64_t pd_wave_frames(const pd_decoder *D, int in_dtype) { return D ? wave_frames(D, in_dtype, nullptr) : 0; }
+int64_t pd_wave_frames(const pd_decoder *D, int in_dtype) { return D ? wave_frames(D, route(D, in_dtype, nullptr)) : 0; }
 int pd_code_len(const pd_decoder *D) { return D ? D->dev.N : 0; }
-const char *pd_kernel_name(const pd_decoder *D) { return D ? D->kernel_name : ""; }
+// the kernel of a call with the decoder's natural input: bytes for the LUT classes, fp64 LLRs for the others
+const char *pd_kernel_name(const pd_decoder *D) { return D ? kRouteName[(int)route(D, D->dev.domain == DOM_LUT ? PD_U8 : PD_F64, nullptr)] : ""; }
 const char *pd_kernel_note(const pd_decoder *D) { return (D && !D->fast.ok && D->dev.domain == DOM_LUT) ? D->fast.why : ""; }
 
 int pd_schedule_stats(const pd_decoder *D, int64_t *n_steps, int64_t *elem_ops, int64_t *n_sorts) {
@@ -845,25 +841,21 @@ int pd_decode_device(pd_decoder *D, const void *dev_in, int in_dtype, int64_t B,
     // events: the CTAs of piece k+1 move into the slots that the CTAs of piece k vacate, so nothing idles between pieces.
     // POLAR_B200_FORCE_SPLIT=0/1 overrides, POLAR_B200_PIECE_WAVES sets the piece size.
     const size_t esz = dtype_size(in_dtype), N = D->dev.N, Ko = D->dev.Kout;
-    const int64_t wave = wave_frames(D, in_dtype, dev_in);
+    const Route r = route(D, in_dtype, dev_in);
+    const int64_t wave = wave_frames(D, r);
     static const int force_split = getenv("POLAR_B200_FORCE_SPLIT") ? atoi(getenv("POLAR_B200_FORCE_SPLIT")) : -1;
     static const int piece_waves = getenv("POLAR_B200_PIECE_WAVES") ? std::max(1, atoi(getenv("POLAR_B200_PIECE_WAVES"))) : 1;
-    const bool dynamic_kernel = want_fast(D, in_dtype, dev_in) && !D->fast.fastk;
+    const bool dynamic_kernel = r == Route::Lut && !D->fast.fastk;
     const bool split = force_split == 0 ? false
                                         : ((force_split == 1 || !dynamic_kernel) && wave > 0 && B >= 2 * wave * piece_waves && ((N * esz) % 16 == 0));
     const int64_t per = split ? wave * piece_waves : B;
     const int pieces = split ? (int)((B + per - 1) / per) : 1;
     // workspace: one region per concurrently running piece
-    const size_t need1 = ws_need(D, in_dtype, dev_in, per);
+    const size_t need1 = ws_need(D, r, per);
     const size_t need = need1 * (split ? 2 : 1);
-    if (need > D->ws_user_cap) {
-        CUDA_TRY(cudaDeviceSynchronize());
-        cudaFree(D->ws_user);
-        D->ws_user = nullptr; D->ws_user_cap = 0;
-        CUDA_TRY(cudaMalloc((void **)&D->ws_user, need));
-        D->ws_user_cap = need;
-    }
-    if (!split) return launch(D, dev_in, in_dtype, B, dev_out, s, D->ws_user);
+    if (need > D->ws_user_cap) CUDA_TRY(cudaDeviceSynchronize());   // launches in flight may still use the old workspace
+    CUDA_TRY(grow(&D->ws_user, &D->ws_user_cap, need));
+    if (!split) return launch(D, r, dev_in, in_dtype, B, dev_out, s, D->ws_user);
     if (!D->fork_ev) {
         CUDA_TRY(cudaEventCreateWithFlags(&D->fork_ev, cudaEventDisableTiming));
         for (int i = 0; i < 2; ++i) {
@@ -880,7 +872,7 @@ int pd_decode_device(pd_decoder *D, const void *dev_in, int in_dtype, int64_t B,
         const int64_t f0 = (int64_t)pc * per, nb = std::min<int64_t>(per, B - f0);
         if (nb <= 0) break;
         const int w = pc & 1;
-        if ((rc = launch(D, (const char *)dev_in + (size_t)f0 * N * esz, in_dtype, nb, dev_out + (size_t)f0 * Ko, D->side[w],
+        if ((rc = launch(D, r, (const char *)dev_in + (size_t)f0 * N * esz, in_dtype, nb, dev_out + (size_t)f0 * Ko, D->side[w],
                          D->ws_user ? D->ws_user + (size_t)w * need1 : nullptr)))
             return rc;
     }
@@ -905,70 +897,50 @@ int pd_check(pd_decoder *D, void *cuda_stream) {
 // ---- blind-detection kinds ------------------------------------------------------------------------
 int pd_decode_bd_device(pd_decoder *D, const double *dev_llr, int64_t B, const int32_t *dev_rnti, int32_t rnti_len,
                         uint8_t *dev_bits, double *dev_metric, uint8_t *dev_pass, void *cuda_stream) {
-    if (!D || (B > 0 && (!dev_llr || !dev_metric))) return fail(PD_EINVAL, "null argument");
-    if (D->dev.bd == 0) return fail(PD_EINVAL, "pd_decode_bd: the decoder is not a PD_BD_* kind");
-    if (D->dev.bd == 2) {
-        if (B > 0 && (!dev_bits || !dev_pass)) return fail(PD_EINVAL, "null argument");
-        if (rnti_len < 0 || rnti_len > D->dev.crc_n || (rnti_len > 0 && !dev_rnti)) return fail(PD_EINVAL, "RNTI length %d must be in [0,crc_n=%d]", rnti_len, D->dev.crc_n);
-    }
-    if (B <= 0) return PD_OK;
+    const int rc0 = check_bd(D, dev_llr, B, dev_rnti, rnti_len, dev_bits, dev_metric, dev_pass);
+    if (rc0 || B <= 0) return rc0;
     CUDA_TRY(cudaSetDevice(D->device));
     cudaStream_t s = (cudaStream_t)cuda_stream;
-    const size_t need = ws_need(D, PD_F64, dev_llr, B);
-    if (need > D->ws_user_cap) {
-        CUDA_TRY(cudaDeviceSynchronize());
-        cudaFree(D->ws_user);
-        D->ws_user = nullptr; D->ws_user_cap = 0;
-        CUDA_TRY(cudaMalloc((void **)&D->ws_user, need));
-        D->ws_user_cap = need;
-    }
+    const Route r = route(D, PD_F64, dev_llr);
+    const size_t need = ws_need(D, r, B);
+    if (need > D->ws_user_cap) CUDA_TRY(cudaDeviceSynchronize());   // launches in flight may still use the old workspace
+    CUDA_TRY(grow(&D->ws_user, &D->ws_user_cap, need));
     // per-call pointers ride in the descriptor, which every launch copies by value
     Dev &d = D->dev;
     d.bd_rnti = dev_rnti; d.bd_rnti_len = d.bd == 2 ? rnti_len : 0; d.bd_metric = dev_metric; d.bd_pass = dev_pass;
-    const int rc = launch(D, dev_llr, PD_F64, B, d.bd == 2 ? dev_bits : nullptr, s, D->ws_user);
+    const int rc = launch(D, r, dev_llr, PD_F64, B, d.bd == 2 ? dev_bits : nullptr, s, D->ws_user);
     d.bd_rnti = nullptr; d.bd_rnti_len = 0; d.bd_metric = nullptr; d.bd_pass = nullptr;
     return rc;
 }
 
 int pd_decode_bd(pd_decoder *D, const double *llr, int64_t B, const int32_t *rnti, int32_t rnti_len,
                  uint8_t *out_bits, double *out_metric, uint8_t *out_pass) {
-    if (!D || (B > 0 && (!llr || !out_metric))) return fail(PD_EINVAL, "null argument");
-    if (D->dev.bd == 0) return fail(PD_EINVAL, "pd_decode_bd: the decoder is not a PD_BD_* kind");
-    const bool ca = D->dev.bd == 2;
-    if (ca && B > 0 && (!out_bits || !out_pass)) return fail(PD_EINVAL, "null argument");
-    if (ca && (rnti_len < 0 || rnti_len > D->dev.crc_n || (rnti_len > 0 && !rnti))) return fail(PD_EINVAL, "RNTI length %d must be in [0,crc_n=%d]", rnti_len, D->dev.crc_n);
-    if (B <= 0) return PD_OK;
+    int rc = check_bd(D, llr, B, rnti, rnti_len, out_bits, out_metric, out_pass);
+    if (rc || B <= 0) return rc;
     CUDA_TRY(cudaSetDevice(D->device));
+    const bool ca = D->dev.bd == 2;
     const size_t N = D->dev.N, Ko = D->dev.Kout;
     const int64_t chunk = std::min<int64_t>(B, std::max<int64_t>(1024, (int64_t)((32u << 20) / (N * 8))));
-    double *d_in = nullptr, *d_metric = nullptr;
-    uint8_t *d_bits = nullptr, *d_pass = nullptr;
-    int32_t *d_rnti = nullptr;
-    int rc = PD_OK;
-    auto cleanup = [&]() { cudaFree(d_in); cudaFree(d_metric); cudaFree(d_bits); cudaFree(d_pass); cudaFree(d_rnti); };
-    if (cudaMalloc((void **)&d_in, (size_t)chunk * N * 8) != cudaSuccess || cudaMalloc((void **)&d_metric, (size_t)chunk * 8) != cudaSuccess ||
-        cudaMalloc((void **)&d_bits, std::max<size_t>((size_t)chunk * Ko, 16)) != cudaSuccess || cudaMalloc((void **)&d_pass, (size_t)chunk) != cudaSuccess ||
-        cudaMalloc((void **)&d_rnti, std::max<size_t>((size_t)rnti_len * 4, 16)) != cudaSuccess) {
-        cleanup();
-        cudaGetLastError();
-        return fail(PD_ENOMEM, "cudaMalloc failed");
-    }
+    DevBufs b;
+    double *d_in = b.get<double>((size_t)chunk * N), *d_metric = b.get<double>(chunk);
+    uint8_t *d_bits = b.get<uint8_t>((size_t)chunk * Ko), *d_pass = b.get<uint8_t>(chunk);
+    int32_t *d_rnti = b.get<int32_t>((size_t)rnti_len);
+    if (!d_in || !d_metric || !d_bits || !d_pass || !d_rnti) return fail(PD_ENOMEM, "cudaMalloc failed");
     cudaStream_t s = nullptr;
-    if (ca && rnti_len > 0 && cudaMemcpyAsync(d_rnti, rnti, (size_t)rnti_len * 4, cudaMemcpyHostToDevice, s) != cudaSuccess) rc = fail(PD_ECUDA, "H2D copy failed");
-    for (int64_t f0 = 0; f0 < B && rc == PD_OK; f0 += chunk) {
+    if (ca && rnti_len > 0 && cudaMemcpyAsync(d_rnti, rnti, (size_t)rnti_len * 4, cudaMemcpyHostToDevice, s) != cudaSuccess) return fail(PD_ECUDA, "H2D copy failed");
+    for (int64_t f0 = 0; f0 < B; f0 += chunk) {
         const int64_t nb = std::min<int64_t>(chunk, B - f0);
-        if (cudaMemcpyAsync(d_in, llr + (size_t)f0 * N, (size_t)nb * N * 8, cudaMemcpyHostToDevice, s) != cudaSuccess) { rc = fail(PD_ECUDA, "H2D copy failed"); break; }
-        if ((rc = pd_decode_bd_device(D, d_in, nb, d_rnti, rnti_len, d_bits, d_metric, d_pass, s))) break;
+        if (cudaMemcpyAsync(d_in, llr + (size_t)f0 * N, (size_t)nb * N * 8, cudaMemcpyHostToDevice, s) != cudaSuccess) return fail(PD_ECUDA, "H2D copy failed");
+        if ((rc = pd_decode_bd_device(D, d_in, nb, d_rnti, rnti_len, d_bits, d_metric, d_pass, s))) return rc;
         bool ok = cudaMemcpyAsync(out_metric + f0, d_metric, (size_t)nb * 8, cudaMemcpyDeviceToHost, s) == cudaSuccess;
         if (ca) {
             ok = ok && cudaMemcpyAsync(out_bits + (size_t)f0 * Ko, d_bits, (size_t)nb * Ko, cudaMemcpyDeviceToHost, s) == cudaSuccess;
             ok = ok && cudaMemcpyAsync(out_pass + f0, d_pass, (size_t)nb, cudaMemcpyDeviceToHost, s) == cudaSuccess;
         }
-        if (!ok) { rc = fail(PD_ECUDA, "D2H copy failed"); break; }
-        rc = pd_check(D, s);
+        if (!ok) return fail(PD_ECUDA, "D2H copy failed");
+        if ((rc = pd_check(D, s))) return rc;
     }
-    cleanup();
-    return rc;
+    return PD_OK;
 }
 
 int pd_decode(pd_decoder *D, const void *host_in, int in_dtype, int64_t B, uint8_t *host_out) {
@@ -989,14 +961,14 @@ int pd_decode(pd_decoder *D, const void *host_in, int in_dtype, int64_t B, uint8
             D->h_small = (char *)hp; D->d_small = (char *)dp;
         }
         const int small_dtype = f64_symbols ? PD_U8 : in_dtype;
-        const size_t wsn = std::max(ws_need(D, small_dtype, D->d_small, B), (size_t)16);
-        if (sl.ws_cap < wsn) { cudaFree(sl.ws); sl.ws = nullptr; sl.ws_cap = 0; CUDA_TRY(cudaMalloc((void **)&sl.ws, wsn)); sl.ws_cap = wsn; }
+        const Route r = route(D, small_dtype, D->d_small);
+        CUDA_TRY(grow(&sl.ws, &sl.ws_cap, std::max(ws_need(D, r, B), (size_t)16)));
         if (f64_symbols) {
             if (!narrow_f64_to_u8((const double *)host_in, (uint8_t *)D->h_small, (size_t)B * N)) return fail(PD_ERANGE, "input symbol outside 0..255");
         } else {
             memcpy(D->h_small, host_in, (size_t)B * N * esz);
         }
-        if ((rc = launch(D, D->d_small, small_dtype, B, reinterpret_cast<uint8_t *>(D->d_small + kSmallIn), sl.stream, sl.ws))) return rc;
+        if ((rc = launch(D, r, D->d_small, small_dtype, B, reinterpret_cast<uint8_t *>(D->d_small + kSmallIn), sl.stream, sl.ws))) return rc;
         if ((rc = pd_check(D, sl.stream))) return rc;
         memcpy(host_out, D->h_small + kSmallIn, (size_t)B * Ko);
         return PD_OK;
@@ -1006,11 +978,11 @@ int pd_decode(pd_decoder *D, const void *host_in, int in_dtype, int64_t B, uint8
     // stream slots per unit, so that the copies of one chunk hide behind the kernel of another.
     std::vector<pd_decoder *> units = D->units.empty() ? std::vector<pd_decoder *>{D} : D->units;
     const int U = (int)units.size();
-    const bool narrow = (in_dtype == PD_I32 && D->fast.ok && D->force == 0) || f64_symbols;   // int32 / float64-typed symbols travel as bytes
+    const bool narrow = (in_dtype == PD_I32 && route(D, PD_U8, nullptr) == Route::Lut) || f64_symbols;   // int32 / float64-typed symbols travel as bytes
     const size_t dsz = narrow ? 1 : esz;                                        // element size on the device
     const int dev_dtype = narrow ? PD_U8 : in_dtype;
     int64_t chunk = std::max<int64_t>(8192, (int64_t)((16u << 20) / (N * dsz)));
-    if (const int64_t wave = wave_frames(D, dev_dtype, nullptr)) chunk = std::max<int64_t>(1, (chunk + wave / 2) / wave) * wave;
+    if (const int64_t wave = wave_frames(D, route(D, dev_dtype, nullptr))) chunk = std::max<int64_t>(1, (chunk + wave / 2) / wave) * wave;
     if (const char *e = getenv("POLAR_B200_CHUNK_FRAMES")) chunk = std::max(1, atoi(e));      // (tests: force many small chunks)
     chunk = std::min<int64_t>(B, chunk);
     // the caller's buffers go through pinned staging memory unless they are pinned already (pd_host_alloc / cudaHostRegister):
@@ -1021,14 +993,13 @@ int pd_decode(pd_decoder *D, const void *host_in, int in_dtype, int64_t B, uint8
         for (auto &sl : u->slot) {
             if (!sl.stream) CUDA_TRY(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
             if (!sl.done) CUDA_TRY(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
-            size_t in_need = (size_t)chunk * N * dsz, out_need = (size_t)chunk * Ko;
-            if (sl.in_cap < in_need) { cudaFree(sl.d_in); sl.d_in = nullptr; sl.in_cap = 0; CUDA_TRY(cudaMalloc(&sl.d_in, in_need)); sl.in_cap = in_need; }
-            if (sl.out_cap < out_need) { cudaFree(sl.d_out); sl.d_out = nullptr; sl.out_cap = 0; CUDA_TRY(cudaMalloc((void **)&sl.d_out, out_need)); sl.out_cap = out_need; }
-            if (stage_in && sl.h_in_cap < in_need) { if (sl.h_in) cudaFreeHost(sl.h_in); sl.h_in = nullptr; sl.h_in_cap = 0; CUDA_TRY(cudaHostAlloc((void **)&sl.h_in, in_need, cudaHostAllocPortable)); sl.h_in_cap = in_need; }
-            if (stage_out && sl.h_out_cap < out_need) { if (sl.h_out) cudaFreeHost(sl.h_out); sl.h_out = nullptr; sl.h_out_cap = 0; CUDA_TRY(cudaHostAlloc((void **)&sl.h_out, out_need, cudaHostAllocPortable)); sl.h_out_cap = out_need; }
+            const size_t in_need = (size_t)chunk * N * dsz, out_need = (size_t)chunk * Ko;
+            CUDA_TRY(grow(&sl.d_in, &sl.in_cap, in_need));
+            CUDA_TRY(grow(&sl.d_out, &sl.out_cap, out_need));
+            if (stage_in) CUDA_TRY(grow_pinned(&sl.h_in, &sl.h_in_cap, in_need));
+            if (stage_out) CUDA_TRY(grow_pinned(&sl.h_out, &sl.h_out_cap, out_need));
             // our own staging buffers are cudaMalloc'ed (256-B aligned), so the kernel choice depends on the dtype only
-            size_t wsn = std::max(ws_need(u, dev_dtype, nullptr, chunk), (size_t)16);
-            if (sl.ws_cap < wsn) { cudaFree(sl.ws); sl.ws = nullptr; sl.ws_cap = 0; CUDA_TRY(cudaMalloc((void **)&sl.ws, wsn)); sl.ws_cap = wsn; }
+            CUDA_TRY(grow(&sl.ws, &sl.ws_cap, std::max(ws_need(u, route(u, dev_dtype, nullptr), chunk), (size_t)16)));
         }
     }
     static const bool trace = getenv("POLAR_B200_TRACE") != nullptr;
@@ -1085,7 +1056,7 @@ int pd_decode(pd_decoder *D, const void *host_in, int in_dtype, int64_t B, uint8
         }
         PD_TRACE("chunk at %lld (%lld frames) staged -> slot %d", (long long)f0, (long long)nb, which);
         CUDA_TRY(cudaMemcpyAsync(sl.d_in, h2d_src, (size_t)nb * N * dsz, cudaMemcpyHostToDevice, sl.stream));
-        if ((rc = launch(u, sl.d_in, dev_dtype, nb, sl.d_out, sl.stream, sl.ws))) return rc;
+        if ((rc = launch(u, route(u, dev_dtype, sl.d_in), sl.d_in, dev_dtype, nb, sl.d_out, sl.stream, sl.ws))) return rc;
         PD_TRACE("chunk at %lld launched", (long long)f0);
         CUDA_TRY(cudaMemcpyAsync(stage_out ? (void *)sl.h_out : (void *)(host_out + (size_t)f0 * Ko), sl.d_out, (size_t)nb * Ko, cudaMemcpyDeviceToHost, sl.stream));
         CUDA_TRY(cudaEventRecord(sl.done, sl.stream));
@@ -1181,16 +1152,6 @@ void pd_sim_destroy(pd_sim *S) {
     delete S;
 }
 
-// copies `bytes` host bytes into a new device buffer owned by S (freed by pd_sim_destroy)
-static int sim_upload(pd_sim *S, const void *h, size_t bytes, const void **dst) {
-    void *p = nullptr;
-    if (cudaMalloc(&p, std::max<size_t>(bytes, 16)) != cudaSuccess) return fail(PD_ECUDA, "cudaMalloc failed");
-    S->allocs.push_back(p);
-    if (bytes && cudaMemcpy(p, h, bytes, cudaMemcpyHostToDevice) != cudaSuccess) return fail(PD_ECUDA, "cudaMemcpy failed");
-    *dst = p;
-    return PD_OK;
-}
-
 int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
     if (!c || !out || !c->frozen_bits) return fail(PD_EINVAL, "null argument");
     *out = nullptr;
@@ -1202,25 +1163,18 @@ int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
     if (c->crc_n < 0 || c->crc_n > 32) return fail(PD_EINVAL, "crc_n must be in [0,32]");
     if (c->A < 1 || c->A + c->crc_n != c->K) return fail(PD_EINVAL, "need K == A + crc_n");
     if (c->edges && (c->n_edges < 2 || !c->chan_lut || c->q_channel < 1 || c->q_channel > 256)) return fail(PD_EINVAL, "bad channel quantizer");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(PD_ECUDA, "no CUDA device");
-    if (c->device < 0 || c->device >= ndev) return fail(PD_EINVAL, "device %d out of range", c->device);
-    CUDA_TRY(cudaSetDevice(c->device));
+    const int rc = probe_device(c->device);
+    if (rc) return rc;
     pd_sim *S = new pd_sim();
+    std::unique_ptr<pd_sim, void (*)(pd_sim *)> own(S, pd_sim_destroy);   // frees S on every error return
     S->device = c->device;
     SimDev &d = S->dev;
     d.N = N; d.K = c->K; d.A = c->A; d.crc_n = c->crc_n;
-    int rc;
-    if ((rc = sim_upload(S, info_pos.data(), info_pos.size() * 4, (const void **)&d.info_pos))) { pd_sim_destroy(S); return rc; }
+    CUDA_TRY(upload(S->allocs, info_pos.data(), info_pos.size(), &d.info_pos));
     std::vector<uint32_t> rem(c->A, 0);
     if (c->crc_n > 0) {
-        std::vector<int> poly(c->crc_n + 1, 0);
-        for (int i = 0; i < c->crc_loc_len; ++i) {
-            if (c->crc_loc[i] < 0 || c->crc_loc[i] > c->crc_n) { pd_sim_destroy(S); return fail(PD_EINVAL, "crc_p entry out of range"); }
-            poly[c->crc_loc[i]] = 1;
-        }
         uint32_t taps = 0;
-        for (int k = 0; k < c->crc_n; ++k) if (poly[1 + k]) taps |= 1u << (c->crc_n - 1 - k);
+        if (!crc_taps(c->crc_n, c->crc_loc, c->crc_loc_len, &taps)) return fail(PD_EINVAL, "crc_p entry out of range");
         const uint32_t msb = 1u << (c->crc_n - 1), mask = c->crc_n >= 32 ? 0xffffffffu : ((1u << c->crc_n) - 1u);
         for (int k = 0; k < c->A; ++k) {
             uint32_t reg = 0;
@@ -1232,7 +1186,7 @@ int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
             rem[k] = reg;
         }
     }
-    if ((rc = sim_upload(S, rem.data(), rem.size() * 4, (const void **)&d.crc_rem))) { pd_sim_destroy(S); return rc; }
+    CUDA_TRY(upload(S->allocs, rem.data(), rem.size(), &d.crc_rem));
     if (N <= 1024) {
         std::vector<EncWord> tab(32);
         memset(tab.data(), 0, tab.size() * sizeof(EncWord));
@@ -1245,18 +1199,18 @@ int pd_sim_create(const pd_sim_config *c, pd_sim **out) {
             enc_expand_masks(m, tab[w].mv);
             before += (uint32_t)__builtin_popcount(m);
         }
-        if ((rc = sim_upload(S, tab.data(), tab.size() * sizeof(EncWord), (const void **)&S->enc_tab))) { pd_sim_destroy(S); return rc; }
+        CUDA_TRY(upload(S->allocs, tab.data(), tab.size(), &S->enc_tab));
     }
     if (c->edges) {
-        if ((rc = sim_upload(S, c->edges, (size_t)c->n_edges * 8, (const void **)&d.edges)) ||
-            (rc = sim_upload(S, c->chan_lut, (size_t)(c->n_edges - 1), (const void **)&d.chan_lut))) { pd_sim_destroy(S); return rc; }
+        CUDA_TRY(upload(S->allocs, c->edges, (size_t)c->n_edges, &d.edges));
+        CUDA_TRY(upload(S->allocs, c->chan_lut, (size_t)(c->n_edges - 1), &d.chan_lut));
         d.n_edges = c->n_edges;
         d.q_channel = c->q_channel;
         d.mode = PD_SIM_LLR_QUANT;
     } else {
         d.mode = PD_SIM_LLR;
     }
-    *out = S;
+    *out = own.release();
     return PD_OK;
 }
 
@@ -1293,9 +1247,8 @@ int pd_sim_set_channel(pd_sim *S, const pd_sim_channel *ch) {
         return fail(PD_EINVAL, "unknown channel mode %d", ch->mode);
     }
     CUDA_TRY(cudaSetDevice(S->device));
-    int rc;
-    if (d.n_edges && (rc = sim_upload(S, ch->edges, (size_t)d.n_edges * 8, (const void **)&d.edges))) return rc;
-    if (llr_quant && (rc = sim_upload(S, ch->chan_lut, (size_t)(d.n_edges - 1), (const void **)&d.chan_lut))) return rc;
+    if (d.n_edges) CUDA_TRY(upload(S->allocs, ch->edges, (size_t)d.n_edges, &d.edges));
+    if (llr_quant) CUDA_TRY(upload(S->allocs, ch->chan_lut, (size_t)(d.n_edges - 1), &d.chan_lut));
     S->dev = d;
     return PD_OK;
 }
@@ -1354,20 +1307,17 @@ int pd_sim_encode(pd_sim *S, int mode, const uint8_t *in, int64_t B, uint8_t *ou
     CUDA_TRY(cudaSetDevice(S->device));
     // bounded staging: chunks of <= 32 MiB of output
     const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(B, ((int64_t)32 << 20) / out_len));
-    uint8_t *d_in = nullptr, *d_out = nullptr;
-    if (cudaMalloc(&d_in, (size_t)chunk * in_len) != cudaSuccess) return fail(PD_ENOMEM, "cudaMalloc failed");
-    if (cudaMalloc(&d_out, (size_t)chunk * out_len) != cudaSuccess) { cudaFree(d_in); return fail(PD_ENOMEM, "cudaMalloc failed"); }
-    rc = PD_OK;
-    for (int64_t f0 = 0; f0 < B && rc == PD_OK; f0 += chunk) {
+    DevBufs bufs;
+    uint8_t *d_in = bufs.get<uint8_t>((size_t)chunk * in_len), *d_out = bufs.get<uint8_t>((size_t)chunk * out_len);
+    if (!d_in || !d_out) return fail(PD_ENOMEM, "cudaMalloc failed");
+    for (int64_t f0 = 0; f0 < B; f0 += chunk) {
         const int64_t b = std::min(chunk, B - f0);
-        if (cudaMemcpyAsync(d_in, in + (size_t)f0 * in_len, (size_t)b * in_len, cudaMemcpyHostToDevice, 0) != cudaSuccess) { rc = fail(PD_ECUDA, "H2D copy failed"); break; }
-        if ((rc = pd_sim_encode_device(S, mode, d_in, b, d_out, nullptr))) break;
-        if (cudaMemcpyAsync(out + (size_t)f0 * out_len, d_out, (size_t)b * out_len, cudaMemcpyDeviceToHost, 0) != cudaSuccess) { rc = fail(PD_ECUDA, "D2H copy failed"); break; }
-        if (cudaStreamSynchronize(0) != cudaSuccess) { rc = fail(PD_ECUDA, "encode failed: %s", cudaGetErrorString(cudaGetLastError())); break; }
+        if (cudaMemcpyAsync(d_in, in + (size_t)f0 * in_len, (size_t)b * in_len, cudaMemcpyHostToDevice, 0) != cudaSuccess) return fail(PD_ECUDA, "H2D copy failed");
+        if ((rc = pd_sim_encode_device(S, mode, d_in, b, d_out, nullptr))) return rc;
+        if (cudaMemcpyAsync(out + (size_t)f0 * out_len, d_out, (size_t)b * out_len, cudaMemcpyDeviceToHost, 0) != cudaSuccess) return fail(PD_ECUDA, "D2H copy failed");
+        if (cudaStreamSynchronize(0) != cudaSuccess) return fail(PD_ECUDA, "encode failed: %s", cudaGetErrorString(cudaGetLastError()));
     }
-    cudaFree(d_in);
-    cudaFree(d_out);
-    return rc;
+    return PD_OK;
 }
 
 // ---- lookup-table design: batched minimum-distortion quantizer -----------------------------------------
@@ -1383,66 +1333,42 @@ int pd_optls_quantize(const double *density, const double *quanta, const int32_t
             if (!(quanta[(size_t)p * stride + i] > quanta[(size_t)p * stride + i - 1])) return fail(PD_EINVAL, "problem %d: quanta must be strictly ascending (pass np.unique output)", p);
         maxM = std::max(maxM, M[p]);
     }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(PD_ECUDA, "no CUDA device: libpolar_b200 has no CPU path");
-    if (device < 0 || device >= ndev) return fail(PD_EINVAL, "device %d out of range", device);
-    CUDA_TRY(cudaSetDevice(device));
+    const int rc = probe_device(device);
+    if (rc) return rc;
     const int W = maxM - K + 1;
     const long long t_stride = (long long)maxM * W, lm_stride = (long long)(K + 1) * W;
     const int chunk = (int)std::max<long long>(1, std::min<long long>(P, (256ll << 20) / (t_stride * 8)));   // <= 256 MiB of tables in flight
-    double *d_d = nullptr, *d_q = nullptr, *d_od = nullptr, *d_oq = nullptr, *d_T = nullptr;
-    int32_t *d_M = nullptr, *d_lut = nullptr, *d_lm = nullptr;
-    auto cleanup = [&]() { cudaFree(d_d); cudaFree(d_q); cudaFree(d_od); cudaFree(d_oq); cudaFree(d_T); cudaFree(d_M); cudaFree(d_lut); cudaFree(d_lm); };
-    if (cudaMalloc((void **)&d_d, (size_t)chunk * stride * 8) != cudaSuccess || cudaMalloc((void **)&d_q, (size_t)chunk * stride * 8) != cudaSuccess ||
-        cudaMalloc((void **)&d_od, (size_t)chunk * K * 8) != cudaSuccess || cudaMalloc((void **)&d_oq, (size_t)chunk * K * 8) != cudaSuccess ||
-        cudaMalloc((void **)&d_T, (size_t)chunk * t_stride * 8) != cudaSuccess || cudaMalloc((void **)&d_M, (size_t)chunk * 4) != cudaSuccess ||
-        cudaMalloc((void **)&d_lut, (size_t)chunk * stride * 4) != cudaSuccess || cudaMalloc((void **)&d_lm, (size_t)chunk * lm_stride * 4) != cudaSuccess) {
-        cleanup();
-        cudaGetLastError();
-        return fail(PD_ENOMEM, "cudaMalloc failed");
-    }
-    int rc = PD_OK;
+    DevBufs b;
+    double *d_d = b.get<double>((size_t)chunk * stride), *d_q = b.get<double>((size_t)chunk * stride);
+    double *d_od = b.get<double>((size_t)chunk * K), *d_oq = b.get<double>((size_t)chunk * K), *d_T = b.get<double>((size_t)chunk * t_stride);
+    int32_t *d_M = b.get<int32_t>(chunk), *d_lut = b.get<int32_t>((size_t)chunk * stride), *d_lm = b.get<int32_t>((size_t)chunk * lm_stride);
+    if (!d_d || !d_q || !d_od || !d_oq || !d_T || !d_M || !d_lut || !d_lm) return fail(PD_ENOMEM, "cudaMalloc failed");
     const size_t smem = (size_t)(2 * maxM + 2 * W) * sizeof(double);
-    for (int p0 = 0; p0 < P && rc == PD_OK; p0 += chunk) {
+    for (int p0 = 0; p0 < P; p0 += chunk) {
         const int np = std::min(chunk, P - p0);
         bool ok = cudaMemcpy(d_d, density + (size_t)p0 * stride, (size_t)np * stride * 8, cudaMemcpyHostToDevice) == cudaSuccess &&
                   cudaMemcpy(d_q, quanta + (size_t)p0 * stride, (size_t)np * stride * 8, cudaMemcpyHostToDevice) == cudaSuccess &&
                   cudaMemcpy(d_M, M + p0, (size_t)np * 4, cudaMemcpyHostToDevice) == cudaSuccess;
-        if (!ok) { rc = fail(PD_ECUDA, "H2D copy failed"); break; }
+        if (!ok) return fail(PD_ECUDA, "H2D copy failed");
         const cudaError_t le = launch_optls(np, smem, d_d, d_q, d_M, stride, K, d_od, d_oq, d_lut, d_T, d_lm, t_stride, lm_stride);
         g_launches++;
         ok = le == cudaSuccess &&
              cudaMemcpy(out_density + (size_t)p0 * K, d_od, (size_t)np * K * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
              cudaMemcpy(out_quanta + (size_t)p0 * K, d_oq, (size_t)np * K * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
              cudaMemcpy(out_lut + (size_t)p0 * stride, d_lut, (size_t)np * stride * 4, cudaMemcpyDeviceToHost) == cudaSuccess;
-        if (!ok) rc = fail(PD_ECUDA, "optls kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
+        if (!ok) return fail(PD_ECUDA, "optls kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
     }
-    cleanup();
-    return rc;
+    return PD_OK;
 }
 
 // ---- lookup-table design, probability domain: the two device passes of the MMI quantizer (see pb_lutgen.cuh) --------
 }  // extern "C"
 namespace {
-struct DevBufs {
-    std::vector<void *> v;
-    ~DevBufs() { for (void *p : v) cudaFree(p); }
-    template <class T> T *get(size_t n) {
-        void *p = nullptr;
-        if (cudaMalloc(&p, std::max<size_t>(n * sizeof(T), 16)) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        v.push_back(p);
-        return reinterpret_cast<T *>(p);
-    }
-};
 int mmi_check(const void *a, const void *b, int32_t P, int32_t M, int32_t K, int32_t device) {
     if (!a || !b) return fail(PD_EINVAL, "null argument");
     if (K < 2 || K > 64 || M < K || M > kOptlsMaxM) return fail(PD_EINVAL, "need 2 <= K <= 64 and K <= M <= %d (K=%d, M=%d)", kOptlsMaxM, K, M);
     if ((long long)P * M * (M - K + 1) > (1ll << 27)) return fail(PD_EINVAL, "too many problems in one call (P*M*(M-K+1) <= 2^27)");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(PD_ECUDA, "no CUDA device: libpolar_b200 has no CPU path");
-    if (device < 0 || device >= ndev) return fail(PD_EINVAL, "device %d out of range", device);
-    CUDA_TRY(cudaSetDevice(device));
-    return PD_OK;
+    return probe_device(device);
 }
 }  // namespace
 extern "C" {

@@ -16,6 +16,10 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <math_constants.h>
+
+#include <algorithm>
+#include <vector>
+
 #include "pb_internal.h"
 
 namespace pb {
@@ -623,5 +627,64 @@ generic_decode_kernel(const Dev d, const void *__restrict__ in, int in_dtype, ui
 }
 
 const void *generic_kernel_fn(int dom, bool list, bool warp);   // instantiations: pb_kernels.cu
+
+// ------------------------------------------------------------------------------------------------
+// host side
+
+// Copies n elements of h into a new device buffer (at least 16 bytes) and records it in `allocs`, whose owner frees it.
+template <typename T>
+inline cudaError_t upload(std::vector<void *> &allocs, const T *h, size_t n, const T **out) {
+    void *p = nullptr;
+    cudaError_t e = cudaMalloc(&p, std::max<size_t>(n * sizeof(T), 16));
+    if (e != cudaSuccess) return e;
+    allocs.push_back(p);
+    if (n && (e = cudaMemcpy(p, h, n * sizeof(T), cudaMemcpyHostToDevice)) != cudaSuccess) return e;
+    *out = reinterpret_cast<const T *>(p);
+    return cudaSuccess;
+}
+
+struct GenericPlan {
+    int threads = 32;
+    size_t ws_bytes = 0;   // per-CTA workspace
+    int use_smem = 0;      // the workspace lives in dynamic shared memory, else in global memory
+    int ctas_per_sm = 1;
+};
+
+// Block size and workspace of the CTA-per-frame kernel; ctas_per_sm < 1 when it does not fit on the device.
+inline cudaError_t plan_generic(const Dev &d, GenericPlan *pl) {
+    const int L = d.list ? d.L : 1;
+    const size_t vsz = d.domain == DOM_LUT ? 1 : 8;
+    size_t ws = (((size_t)L * d.N * vsz + 15) & ~(size_t)15) + (size_t)L * d.r1_tmax * (8 + 4) + (size_t)L * 3 * d.N + (size_t)2 * L * d.r1_tmax + d.N;
+    ws = (ws + 15) & ~(size_t)15;
+    pl->ws_bytes = ws;
+    const int64_t work = (int64_t)L * d.N / 2;
+    int th = 32;
+    while (th < 256 && th * 8 < work) th *= 2;
+    pl->threads = th;
+    pl->use_smem = ws <= 96 * 1024;
+    const void *fn = generic_kernel_fn(d.domain, d.list != 0, th == 32);
+    // (the attribute belongs to the kernel function, which every decoder of the same domain shares: always the cap, never
+    //  this decoder's own size -- a smaller decoder created later must not shrink it under a live larger one)
+    if (pl->use_smem) {
+        const cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&pl->ctas_per_sm, fn, th, pl->use_smem ? ws : 0);
+}
+
+inline int generic_grid(const GenericPlan &pl, long long B, int sm_count) {
+    return (int)std::max<long long>(1, std::min<long long>((long long)sm_count * pl.ctas_per_sm, B));
+}
+
+inline int launch_generic(const Dev &d, const GenericPlan &pl, const void *d_in, int dtype, long long B, uint8_t *d_out,
+                          cudaStream_t s, char *ws, int *d_err, double *dbg_pm, int *dbg_win, int sm_count) {
+    const int grid = generic_grid(pl, B, sm_count);
+    void *args[] = {(void *)&d, (void *)&d_in, (void *)&dtype, (void *)&d_out, (void *)&B, (void *)&ws, (void *)&pl.ws_bytes,
+                    (void *)&pl.use_smem, (void *)&d_err, (void *)&dbg_pm, (void *)&dbg_win};
+    cudaError_t e = cudaLaunchKernel(generic_kernel_fn(d.domain, d.list != 0, pl.threads == 32), dim3(grid), dim3(pl.threads), args,
+                                     pl.use_smem ? pl.ws_bytes : 0, s);
+    if (e != cudaSuccess) return (int)e;
+    return (int)cudaGetLastError();
+}
 
 }  // namespace pb

@@ -85,7 +85,6 @@ struct FastParams {
 struct FastPlan {
     bool ok = false;
     const char *why = "";  // when !ok for a LUT class: which shape rule sent it to the slower kernels
-    const char *name = "generic";
     int logL = 0;
     bool ca = false;
     bool fastk = false;   // the walk contains Fast-SSC special nodes
@@ -1119,16 +1118,6 @@ inline void free_fast_plan(FastPlan *p) {
     p->ok = false;
 }
 
-template <typename T>
-inline bool fast_upload(FastPlan *pl, const std::vector<T> &h, const T **out) {
-    void *p = nullptr;
-    if (cudaMalloc(&p, std::max<size_t>(h.size() * sizeof(T), 16)) != cudaSuccess) return false;
-    pl->allocs.push_back(p);
-    if (!h.empty() && cudaMemcpy(p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice) != cudaSuccess) return false;
-    *out = reinterpret_cast<const T *>(p);
-    return true;
-}
-
 // Kernel instantiations live in their own translation units (pb_kernels.cu, compiled in parallel); the host side only
 // sees the dispatcher.
 const void *fast_kernel_fn(int logL, bool ca, bool fast);
@@ -1410,7 +1399,10 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
     if (P.n_chunks < 1) return;
     std::vector<uint32_t> fw((N + 31) / 32, 0);
     for (int i = 0; i < N; ++i) if (frozen[i] == 1) fw[i >> 5] |= 1u << (i & 31);
-    if (!fast_upload(pl, stream, &P.stream) || !fast_upload(pl, fw, &P.frozen_words)) { free_fast_plan(pl); return; }
+    if (upload(pl->allocs, stream.data(), stream.size(), &P.stream) || upload(pl->allocs, fw.data(), fw.size(), &P.frozen_words)) {
+        free_fast_plan(pl);
+        return;
+    }
     if (d.ca) {
         // remainder of the unit message e_k under the reference's long division (utils.cpp:77-93): linear, so the
         // CRC of a word is the XOR of the remainders of its set bits
@@ -1425,7 +1417,7 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
             }
             rem[k] = reg;
         }
-        if (!fast_upload(pl, rem, &P.crc_rem)) { free_fast_plan(pl); return; }
+        if (upload(pl->allocs, rem.data(), rem.size(), &P.crc_rem)) { free_fast_plan(pl); return; }
         uint32_t cm = 0;
         for (int k = 0; k < d.crc_check; ++k) cm |= 1u << (d.crc_n - 1 - k);
         P.crc_checkmask = cm;
@@ -1476,7 +1468,6 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
     pl->smem = smem_for(best_w);
     pl->ws_bytes_per_cta = (size_t)P.gwords * 32 * 4 * best_w;
     pl->ctas_per_sm = best_occ;
-    pl->name = "scl_lut_warp";
     pl->ok = true;
 }
 
