@@ -855,9 +855,14 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
                 // a*2 + (b>>3) = ((p&15)<<1) | (p>>7), the nibble shift (b&7)*4 = (p>>2) & 0x1c -- for four pairs at once with
                 // byte-lane arithmetic.  w3 = 4 pair bytes of the subtree root, w21 = [15:0] 2 pair bytes of the depth
                 // top+1 node, [23:16] the pair byte of the depth top+2 node, xb = partial sums in place.
+                // SUB16 arg bit h: the half's 8 leaves are all frozen (plan_fast_lut).  Every decision and so every u of
+                // such a half is 0: at L = 1 nothing of it is read (no lines in the stream), at L > 1 it is a
+                // feed-forward map from w3 to 8 leaf LLRs and only the path-metric updates stay serial.
                 xb = 0;
 #pragma unroll 1
                 for (int h = 0; h < (FAST ? 1 : 2); ++h) {
+                    const bool rate0 = !FAST && ((oa >> h) & 1);
+                    if (L == 1 && rate0) { xb <<= 8; continue; }
                     const int s = FAST ? (int)onode : 2 * (int)onode + h;
                     const uint32_t fz = (__ldg(fp.frozen_words + (s >> 2)) >> ((s & 3) * 8)) & 0xffu;
                     {
@@ -866,9 +871,9 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
                             w = *level_ptr(top, vslot(top));
                         } else {
                             // the node's lines end the chunk before each SUB8 part: [.. f] (left half; the chunk may be
-                            // the current one) and [- - g0 g1] (right half; the left part has used its chunks up).
-                            // f is g with t1 = t0 and u = 0.
-                            if (ls.q == 4) ls.cur = next_chunk();
+                            // the current one) and [- - g0 g1] (right half; it is the current chunk when the left half
+                            // left lines in it).  f is g with t1 = t0 and u = 0.
+                            if (ls.q > 3 - h) ls.cur = next_chunk();
                             const uint32_t t1 = ls.cur.w, t0 = h ? ls.cur.z : t1;
                             const uint32_t *src = level_ptr(top - 1, vslot(top - 1));
                             w = lookup8(src[0], src[32], xb, t0, t1, std::true_type{});
@@ -879,9 +884,52 @@ scl_lut_warp_kernel(const __grid_constant__ Dev d, const __grid_constant__ FastP
                         hi = (hi | (hi << 8)) & 0x00ff00ffu; hi = (hi | (hi << 4)) & 0x0f0f0f0fu;
                         w3 = lo | (hi << 4);
                     }
-                    ls.q = 4;
                     auto pb_lane = [](uint32_t P) -> uint32_t { return ((P & 0x0f0f0f0fu) << 1) | ((P >> 7) & 0x01010101u); };
                     auto pb_amt = [](uint32_t P) -> uint32_t { return (P >> 2) & 0x1c1c1c1cu; };
+                    if (!FAST && L > 1 && rate0) {
+                        // all-frozen half: node A (depth top), B0 B1, C0..C3 (depth top+2), each through its f and g0
+                        // tables; pair byte k of P goes through table t_k.  Six chunks [A.f A.g0 B0.f B0.g0]
+                        // [B1.f B1.g0 C0.f C0.g0] [C1.f C1.g0 C2.f C2.g0] [C3.f C3.g0 llr0 llr1] [llr2 .. llr5]
+                        // [llr6 llr7 . .]: the last one stays `cur`, its .z .w are the next lines of the stream.
+                        auto look4 = [&](uint32_t P, uint32_t t0, uint32_t t1, uint32_t t2, uint32_t t3) -> uint32_t {
+                            const uint32_t S = pb_lane(P), H = pb_amt(P);
+                            uint32_t R = 0;
+#pragma unroll
+                            for (int k = 0; k < 4; ++k) {
+                                const uint32_t sel = k == 0 ? 0x3214u : k == 1 ? 0x3240u : k == 2 ? 0x3410u : 0x4210u;
+                                const uint32_t wv = __shfl_sync(kFull, k == 0 ? t0 : k == 1 ? t1 : k == 2 ? t2 : t3, (int)(S >> (8 * k)));
+                                R = __byte_perm(R, __funnelshift_r(wv, 0u, H >> (8 * k)), sel);
+                            }
+                            return R & 0x0f0f0f0fu;    // output k in byte k
+                        };
+                        auto leaf = [&](uint32_t lr, uint32_t sym) {   // (PD/src/SCLLUTDecoder.cpp:92-145, frozen leaf)
+                            const double DM = llr_of(lr, sym & 15u);
+                            if (DM < 0) PM += fabs(DM);
+                        };
+                        uint4 c0, c1;
+                        ring_next_pair(ls.cc, ls.fetch, ring_lane, stream_lane, c0, c1);
+                        const uint32_t fa = look4(w3, c0.x, c0.x, c0.x, c0.x), ga = look4(w3, c0.y, c0.y, c0.y, c0.y);
+                        const uint32_t pb = ((fa | (fa >> 12)) & 0xffffu) | (((ga | (ga >> 12)) & 0xffffu) << 16);   // B0 B0 B1 B1
+                        const uint32_t fb = look4(pb, c0.z, c0.z, c1.x, c1.x), gb = look4(pb, c0.w, c0.w, c1.y, c1.y);
+                        const uint32_t pc = ((fb | (fb >> 4)) & 0x00ff00ffu) | (((gb | (gb >> 4)) & 0x00ff00ffu) << 8);   // C0 C1 C2 C3
+                        const uint32_t c0f = c1.z, c0g = c1.w;
+                        ring_next_pair(ls.cc, ls.fetch, ring_lane, stream_lane, c0, c1);
+                        const uint32_t fc = look4(pc, c0f, c0.x, c0.z, c1.x), gc = look4(pc, c0g, c0.y, c0.w, c1.y);   // leaves 2k, 2k+1
+                        leaf(c1.z, fc);
+                        leaf(c1.w, gc);
+                        ring_next_pair(ls.cc, ls.fetch, ring_lane, stream_lane, c0, c1);
+                        leaf(c0.x, fc >> 8);
+                        leaf(c0.y, gc >> 8);
+                        leaf(c0.z, fc >> 16);
+                        leaf(c0.w, gc >> 16);
+                        leaf(c1.x, fc >> 24);
+                        leaf(c1.y, gc >> 24);
+                        ls.cur = c1;
+                        ls.q = 2;
+                        srt = false;
+                        continue;
+                    }
+                    ls.q = 4;
 #pragma unroll 1
                     for (int c4 = 0; c4 < 4; ++c4) {
                         const int pos = 2 * c4;
@@ -1178,7 +1226,10 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
     //   SPAIR: C.f llr(left) C.g0 C.g1 llr(right)
     //   SUB8 (chunk aligned): per leaf pair c4 two chunks [P0 P1 P2 C.f] [llr C.g0 C.g1 llr] with
     //        (P0,P1,P2) = (A.f,-,B.f) for c4=0, (A.g0,A.g1,B.f) for c4=2, (B.g0,B.g1,-) for c4 odd
-    //   SUB16 (plain walks only): f, the left SUB8's chunks, g0 g1, the right SUB8's chunks; f and g0 g1 end a chunk
+    //   SUB16 (plain walks only): f, the left SUB8's chunks, g0 g1, the right SUB8's chunks; f and g0 g1 end a chunk.
+    //        arg bit h = the 8 leaves of half h are all frozen: at L = 1 the half has no lines at all (nor its f or g0 g1),
+    //        at L > 1 its chunks carry only the f and g0 tables and the LLR rows (push_sub8_rate0), 22 lines, and the
+    //        next op's lines go on in its last chunk
     const int top = n - 3;
     auto heap = [&](int depth, int node) { return (1 << depth) + node - 1; };
     auto push_pad = [&]() { stream.insert(stream.end(), 32, 0u); };
@@ -1256,6 +1307,13 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
             push_llr_row(n - 1, leaf0 + 1);
         }
     };
+    auto push_g0 = [&](int p) { push_table(tabs[p].g_off, tabs[p].g_sz / tabs[p].g_qb, tabs[p].g_qb); };
+    auto push_sub8_rate0 = [&](int node) {   // the lines of an all-frozen one, in the kernel's feed-forward order
+        for (int dd = top; dd <= top + 2; ++dd)
+            for (int k = 0; k < 1 << (dd - top); ++k) { push_f(heap(dd, (node << (dd - top)) + k)); push_g0(heap(dd, (node << (dd - top)) + k)); }
+        for (int j = 0; j < 8; ++j) push_llr_row(n - 1, 8 * node + j);
+    };
+    auto rate0_8 = [&](int node) { for (int j = 0; j < 8; ++j) if (frozen[8 * node + j] != 1) return false; return true; };
     std::function<void(int, int)> walk = [&](int depth, int node) {
         const int p = heap(depth, node), temp = N >> depth;
         const int st = is_special(depth, node);
@@ -1268,11 +1326,15 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
             return;
         }
         if (depth == top - 1 && max_special < 0) {   // plain walk (the plain kernels have no SUB8 case)
-            emit(FOP_SUB16, depth, 0, (uint32_t)node);
-            push_f(p);
-            push_sub8(2 * node);
-            push_g(p);
-            push_sub8(2 * node + 1);
+            const int m = (int)rate0_8(2 * node) | ((int)rate0_8(2 * node + 1) << 1);
+            emit(FOP_SUB16, depth, m, (uint32_t)node);
+            for (int h = 0; h < 2; ++h) {
+                if (L == 1 && ((m >> h) & 1)) continue;
+                if (h == 0) push_f(p);
+                else push_g(p);
+                if ((m >> h) & 1) push_sub8_rate0(2 * node + h);
+                else push_sub8(2 * node + h);
+            }
         } else if (depth < top) {
             emit(FOP_UF, depth, 0, (uint32_t)node); push_f(p);
             walk(depth + 1, 2 * node);
@@ -1366,11 +1428,14 @@ inline void plan_fast_lut(const Dev &d, bool eligible_kind, const int32_t *node_
         const uint32_t oty = ops[i].x & 0xffu;
         auto pad_chunk = [&]() { while ((stream.size() / 32) % 4) stream.insert(stream.end(), 32, 0u); };
         if (oty == FOP_SUB16) {   // [.. f] SUB8 [- - g0 g1] SUB8: the node's lines end the chunk before each SUB8 part
+            const uint32_t m = (ops[i].x >> 16) & 3u;
             auto it = op_lines[i].begin();
             for (int h = 0; h < 2; ++h) {
+                if (L == 1 && ((m >> h) & 1u)) continue;
+                const int sub_lines = ((m >> h) & 1u) ? 22 : 32;
                 while ((stream.size() / 32) % 4 != 3u - h) stream.insert(stream.end(), 32, 0u);
                 stream.insert(stream.end(), it, it + 32 * (1 + h)); it += 32 * (1 + h);
-                stream.insert(stream.end(), it, it + 32 * 32); it += 32 * 32;
+                stream.insert(stream.end(), it, it + 32 * sub_lines); it += 32 * sub_lines;
             }
             continue;
         }
