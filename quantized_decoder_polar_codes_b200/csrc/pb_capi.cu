@@ -517,17 +517,23 @@ Route route(const pd_decoder *D, int dtype, const void *d_in) {
     return Route::Generic;
 }
 
-int launch(pd_decoder *D, Route r, const void *d_in, int dtype, int64_t B, uint8_t *d_out, cudaStream_t s, char *ws) {
+// f0: the frame of the call that is the launch's first frame, so that the debug outputs of a call made of several
+// launches (one-wave pieces, staged chunks) land in the rows of their frames
+int launch(pd_decoder *D, Route r, const void *d_in, int dtype, int64_t B, uint8_t *d_out, cudaStream_t s, char *ws, int64_t f0 = 0) {
     if (B <= 0) return PD_OK;
     const Dev &d = D->dev;
+    // path metrics per frame as the kernel writes them: path_warp rounds L up to a power of two
+    const int64_t pm_stride = r == Route::Path ? (1 << D->path.logL) : d.L;
+    double *dbg_pm = D->dbg_pm ? D->dbg_pm + f0 * pm_stride : nullptr;
+    int *dbg_win = D->dbg_win ? D->dbg_win + f0 : nullptr;
     int rc;
     switch (r) {
-    case Route::Cta: rc = launch_path_cta(d, D->cta, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count); break;
+    case Route::Cta: rc = launch_path_cta(d, D->cta, d_in, dtype, B, d_out, s, ws, D->d_err, dbg_pm, dbg_win, D->sm_count); break;
     case Route::Lut:
-        rc = launch_fast_lut(d, D->fast, d_in, dtype, B, d_out, s, reinterpret_cast<uint32_t *>(ws), D->d_err, D->dbg_pm, D->dbg_win, D->sm_count);
+        rc = launch_fast_lut(d, D->fast, d_in, dtype, B, d_out, s, reinterpret_cast<uint32_t *>(ws), D->d_err, dbg_pm, dbg_win, D->sm_count);
         break;
-    case Route::Path: rc = launch_path_warp(d, D->path, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count); break;
-    default: rc = launch_generic(d, D->generic, d_in, dtype, B, d_out, s, ws, D->d_err, D->dbg_pm, D->dbg_win, D->sm_count); break;
+    case Route::Path: rc = launch_path_warp(d, D->path, d_in, dtype, B, d_out, s, ws, D->d_err, dbg_pm, dbg_win, D->sm_count); break;
+    default: rc = launch_generic(d, D->generic, d_in, dtype, B, d_out, s, ws, D->d_err, dbg_pm, dbg_win, D->sm_count); break;
     }
     g_launches++;
     if (rc != 0) return fail(PD_ECUDA, "%s launch failed: %s", kRouteName[(int)r], cudaGetErrorString((cudaError_t)rc));
@@ -873,7 +879,7 @@ int pd_decode_device(pd_decoder *D, const void *dev_in, int in_dtype, int64_t B,
         if (nb <= 0) break;
         const int w = pc & 1;
         if ((rc = launch(D, r, (const char *)dev_in + (size_t)f0 * N * esz, in_dtype, nb, dev_out + (size_t)f0 * Ko, D->side[w],
-                         D->ws_user ? D->ws_user + (size_t)w * need1 : nullptr)))
+                         D->ws_user ? D->ws_user + (size_t)w * need1 : nullptr, f0)))
             return rc;
     }
     for (int i = 0; i < 2; ++i) {
@@ -1056,7 +1062,7 @@ int pd_decode(pd_decoder *D, const void *host_in, int in_dtype, int64_t B, uint8
         }
         PD_TRACE("chunk at %lld (%lld frames) staged -> slot %d", (long long)f0, (long long)nb, which);
         CUDA_TRY(cudaMemcpyAsync(sl.d_in, h2d_src, (size_t)nb * N * dsz, cudaMemcpyHostToDevice, sl.stream));
-        if ((rc = launch(u, route(u, dev_dtype, sl.d_in), sl.d_in, dev_dtype, nb, sl.d_out, sl.stream, sl.ws))) return rc;
+        if ((rc = launch(u, route(u, dev_dtype, sl.d_in), sl.d_in, dev_dtype, nb, sl.d_out, sl.stream, sl.ws, f0))) return rc;
         PD_TRACE("chunk at %lld launched", (long long)f0);
         CUDA_TRY(cudaMemcpyAsync(stage_out ? (void *)sl.h_out : (void *)(host_out + (size_t)f0 * Ko), sl.d_out, (size_t)nb * Ko, cudaMemcpyDeviceToHost, sl.stream));
         CUDA_TRY(cudaEventRecord(sl.done, sl.stream));

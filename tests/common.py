@@ -29,11 +29,17 @@ TIE_ALPHABET = (-2.0, -1.0, -0.5, 0.0, 0.5, 1.0, 2.0)
 
 
 def make_case(kind, N, K, L=8, A=None, B=64, Q=16, Qc=None, seed=0, tables="random", alphabet=TIE_ALPHABET,
-              per_position=False, share=True, v=16, construction="nr", ebn0_db=2.0, llr_levels=None):
+              per_position=False, share=True, v=16, construction="nr", ebn0_db=2.0, llr_levels=None, frozen=None):
     """Returns (kwargs, x, truth) -- truth is the transmitted info word when the inputs come from a real
-    encode+AWGN chain (tables == "minsum" or the float family with channel=True), else None."""
+    encode+AWGN chain (tables == "minsum" or the float family with channel=True), else None.
+    `frozen` (int mask, 1 = frozen, K zeros) replaces the frozen set of `construction`."""
     rng = np.random.default_rng(seed)
-    fm, mm = sim.frozen_mask(N, K, construction)
+    if frozen is None:
+        fm, mm = sim.frozen_mask(N, K, construction)
+    else:
+        fm = np.asarray(frozen, np.int32)
+        assert fm.shape == (N,) and int((fm == 0).sum()) == K
+        mm = (1 - fm).astype(np.int32)
     kw = dict(N=N, K=K, frozen_bits=fm, message_bits=mm)
     if kind in LIST_KINDS:
         kw["L"] = L

@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 import common
+import fast_walk
 from golden.cases import CASES
 from oracle import polar_oracle as po
 
@@ -53,7 +54,7 @@ BIG = [
     ("SCLLUTDecoder", dict(N=64, K=32, L=5, B=1000)),
     ("SCLLUTDecoder", dict(N=256, K=128, L=16, B=300)),
     ("FastSCLLUTDecoder", dict(N=256, K=128, L=8, B=1500)),
-    ("FastSCLLUTDecoder", dict(N=512, K=300, L=8, B=300)),
+    ("FastSCLLUTDecoder", dict(N=512, K=300, L=8, B=300)),       # an R1 node of 64 leaves at depth 3 -> path_warp
     ("CASCLLUTDecoder", dict(N=128, K=64, L=8, A=40, B=1500)),
     ("CAFastSCLLUTDecoder", dict(N=256, K=128 + 24, L=8, A=128, B=1000)),
     ("SCUniformQuantizedDecoder", dict(N=128, K=64, B=3000)),
@@ -63,7 +64,7 @@ BIG = [
     ("SCLLUTDecoder", dict(N=1024, K=512, L=8, B=300)),
     ("SCLUTDecoder", dict(N=1024, K=512, B=1000)),
     ("CAFastSCLLUTDecoder", dict(N=1024, K=536, A=512, L=8, B=200)),
-    ("FastSCLLUTDecoder", dict(N=1024, K=768, L=8, B=100)),       # high rate: R1 nodes > 32 leaves -> generic kernel
+    ("FastSCLLUTDecoder", dict(N=1024, K=768, L=8, B=100)),       # high rate: R1 nodes > 32 leaves -> path_warp
     ("FastSCLLUTDecoder", dict(N=1024, K=512, L=4, B=200)),
     ("FastSCLLUTDecoder", dict(N=256, K=64, L=2, B=500)),
     ("FastSCLUTDecoder", dict(N=1024, K=700, B=1000)),            # wide R1 / SPC nodes in the non-list warp path
@@ -89,6 +90,9 @@ def test_cuda_matches_oracle(q, kind, ckw, tables):
     kw, x, _ = common.make_case(kind, seed=77, tables=t, ebn0_db=1.0, **ckw)
     want = po.OracleDecoder(kind, **kw).decode(x)
     dec = _build(q, kind, kw)
+    if kind.startswith(("FastSCLUT", "FastSCLLUT", "CAFastSCLLUT")):   # the Fast LUT classes: on scl_lut_warp unless a list R1 node is too wide
+        _, _, eligible, _ = fast_walk.fast_walk(kw["N"], kw["frozen_bits"], kw.get("L", 1))
+        assert dec.kernel == ("scl_lut_warp" if eligible else "path_warp")
     got = dec.decode(x)
     bad = int((got != want).any(axis=1).sum())
     assert bad == 0, f"{bad}/{x.shape[0]} frames differ from the oracle ({dec.kernel})"

@@ -41,7 +41,7 @@ CASES = [
     ("scl_l2", "SCLLUTDecoder", dict(N=64, K=30, L=2, B=40)),
     ("ca_512", "CASCLLUTDecoder", dict(N=512, K=280, A=256, L=8, B=16)),
     ("fastsclut", "FastSCLUTDecoder", dict(N=512, K=256, B=70)),
-    ("fastscl", "FastSCLLUTDecoder", dict(N=512, K=256, L=8, B=16)),
+    ("fastscl", "FastSCLLUTDecoder", dict(N=512, K=256, L=8, B=16)),   # an R1 node of 64 leaves at depth 3: path_warp
     ("cafast", "CAFastSCLLUTDecoder", dict(N=1024, K=536, A=512, L=8, B=8)),
     ("cafast_q", "CAFastSCLLUTDecoder", dict(N=256, K=152, A=128, L=4, B=24, Q=12, Qc=9)),
     ("multi_pass", "SCLLUTDecoder", dict(N=128, K=64, L=8, B=1001)),
